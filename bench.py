@@ -2,6 +2,7 @@
 """bench.py — particle-steps/s of the full SPH + shape-matching + monodomain step (BASELINE.json's metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload 8m|8m_jitter|1m|32m|cfg1|cfg2|<nx>x<ny>x<nz>]
+                    [--dump-outputs DIR]
 
 A "step" is one Animation() of the whole particle set: neighbour search (hash, counting sort = cell table, reorder),
 shape matching (moments, polar decomposition, goal positions), both neighbour passes, ionic model, integration.
@@ -21,6 +22,11 @@ CUDA events on the handle's stream; `cpu_baseline` is the reference's own CPU st
 reference has no threading) on a bounded sample.  With N > 1 the line also carries `mg_parity`: a small lattice stepped
 through the same slab path on all ranks and compared with a single-GPU run on rank 0 before the timed region.  With
 N = 1 and the default workload it carries `also`: quick measurements of the other configurations in the same process.
+
+`--dump-outputs DIR` writes the particle state the timed path left after its last timed step (what a caller reads back
+through Get_Paticles()) as DIR/<field>.npy, so that two builds run with the same arguments can be compared output for output.
+Compare dumps of the same arm only: on a lattice workload the reference arm steps its bounded CPU sample
+(CPU_SAMPLE_DIMS), not the workload the GPU arm steps.
 """
 from __future__ import annotations
 
@@ -58,13 +64,18 @@ WORKLOADS = {
 }
 # BASELINE.json configs[0] / configs[1]: the reference's own particle sets (Resources/*.csv through main.cpp's loader rule,
 # turnOnStim_Mesh), taken from the committed golden fixtures (tests/golden/, generated from the genuine reference by
-# tools/make_golden.py) because /root/reference does not exist on the GPU box.  Small: latency-bound on a GPU; listed for the
-# CPU-vs-GPU comparison on the reference's own inputs, not as the headline.
+# tools/make_golden.py) because the reference's sources are not part of this repository.  Small: latency-bound on a GPU; listed
+# for the CPU-vs-GPU comparison on the reference's own inputs, not as the headline.
 WORKLOADS["cfg1"] = dict(golden="cfg1_4944", quadratic=False, name="Resources/biceps_simple_out_4944.csv, main.cpp defaults (configs[0])")
 WORKLOADS["cfg2"] = dict(golden="cfg2_5211", quadratic=False, name="Resources/biceps_simple_out_18475.csv subsampled to 5211 (configs[1])")
 CPU_SAMPLE_DIMS = (100, 100, 100)  # bounded sample for the CPU legs: a 1M-particle lattice of the same spacing / SM mode (~0.9 s per step)
 CPU_SAMPLE_STEPS = 10              # ~10 s of single-thread CPU work at ~1.2e6 particle-steps/s
 FIXED_WARMUP = 400                 # untimed steps before the timed region, the same for every N (>= 0.1 s under load at N = 8, 0.6 s at N = 1)
+# --dump-outputs: the state a step carries into the next one, i.e. the fields the fast path keeps current (44 B per particle);
+# larger sets are cut to a seeded sample of DUMP_MAX_PARTICLES particles (44 MB)
+DUMP_FIELDS = ("pos", "vel", "dens", "Vm", "Iion", "w", "stim")
+DUMP_MAX_PARTICLES = 1 << 20
+DUMP_SEED = 0
 
 
 def parse_workload(s):
@@ -89,6 +100,18 @@ def make_lattice(dims, jitter=0.0):
     pos, world = inputs.lattice(*dims, jitter=jitter)
     fixed, stim = inputs.lattice_masks(pos, dims[0], 8)
     return pos, world, fixed.astype(np.uint8), np.where(stim, np.float32(300.0), np.float32(0.0)).astype(np.float32)
+
+
+def dump_outputs(out_dir, particles):
+    """DUMP_FIELDS of a Get_Paticles() array as out_dir/<field>.npy (float32, original particle order).  Above
+    DUMP_MAX_PARTICLES particles only a sample is written: the same seeded indices on every run, ascending."""
+    n = len(particles)
+    idx = slice(None)
+    if n > DUMP_MAX_PARTICLES:
+        idx = np.sort(np.random.Generator(np.random.PCG64(DUMP_SEED)).permutation(n)[:DUMP_MAX_PARTICLES])
+    os.makedirs(out_dir, exist_ok=True)
+    for f in DUMP_FIELDS:
+        np.save(os.path.join(out_dir, f + ".npy"), np.ascontiguousarray(particles[f][idx], dtype=np.float32))
 
 
 # ------------------------------------------------------------------------------------------------------------------
@@ -151,9 +174,10 @@ def measured_peak_gbs():
 
 
 # ------------------------------------------------------------------------------------------------------------------
-def cpu_reference_rate(quadratic, steps, warmup, backend=None, wl=None):
+def cpu_reference_rate(quadratic, steps, warmup, backend=None, wl=None, dump_dir=None):
     """The reference's CPU step on this box: genuine class (oracle/_ref, built with its Makefile's -Ofast) when the
-    prebuilt library travelled, else the bit-identical C restatement.  One thread: the reference has no threading."""
+    prebuilt library travelled, else the bit-identical C restatement.  One thread: the reference has no threading.
+    dump_dir: where to write the state after the timed steps (dump_outputs)."""
     from oracle import CpuSim, available_backends
 
     avail = available_backends()
@@ -170,6 +194,8 @@ def cpu_reference_rate(quadratic, steps, warmup, backend=None, wl=None):
     t0 = time.perf_counter()
     sim.Animation(steps)
     dt = time.perf_counter() - t0
+    if dump_dir:
+        dump_outputs(dump_dir, sim.particles())
     kind = "reference" if backend.startswith("ref") else "port"
     flags = {"ref_ofast": "g++ -Ofast (the reference Makefile's flags)", "ref": "g++ -O2 -ffp-contract=off", "port": "gcc -O2 -ffp-contract=off"}[backend]
     d = CPU_SAMPLE_DIMS
@@ -183,9 +209,9 @@ def run_reference(args, wl, rank, world_size):
     if rank != 0:
         return
     whole = "golden" in wl
-    steps = max(1, min(args.steps, 100 if whole else 20))  # each "step" of this arm is one CPU step of the bounded sample (~0.9 s at 1M)
+    steps = args.steps  # each "step" of this arm is one CPU step of the bounded sample (~0.9 s at 1M)
     warmup = min(args.warmup, 100 if whole else 5)
-    base = cpu_reference_rate(wl["quadratic"], steps, warmup, wl=wl)
+    base = cpu_reference_rate(wl["quadratic"], steps, warmup, wl=wl, dump_dir=args.dump_outputs)
     line = {"impl": "reference", "metric": METRIC, "value": base["value"], "unit": UNIT, "n_gpus": args.gpus, "steps": steps,
             "warmup": warmup, "ms_per_step": base["ms_per_step"], "higher_is_better": True, "scaling": "strong",
             "vs_baseline": None, "dtype": "f32", "data": "synthetic",
@@ -416,6 +442,8 @@ def run_ours(args, wl, rank, world_size, local_rank):
     ev_ms = sim.timer_ms()
     clocks = sampler.stop()
     launches = sim.launch_count()
+    if args.dump_outputs:  # after reading the launch count (the download is a launch), before the steps below move the state on
+        dump_outputs(args.dump_outputs, sim.particles())
     t = torch.tensor([ev_ms, wall_ms], dtype=torch.float64, device=f"cuda:{device}")
     if dist is not None:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -571,11 +599,18 @@ def main():
     ap.add_argument("--workload", default="8m")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-also", action="store_true", help="skip the quick measurements of the other configurations (N = 1, default workload)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the particle state after the last timed step as DIR/<field>.npy (float32; a seeded sample of "
+                         f"{DUMP_MAX_PARTICLES} particles for larger sets)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     rank = int(os.environ.get("RANK", "0"))
     world_size = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.dump_outputs and world_size > 1 and args.impl == "ours":
+        ap.error("--dump-outputs needs a single-GPU run: in slab mode each rank holds only its own particles")
     wl = parse_workload(args.workload)
     if args.impl == "reference":
         run_reference(args, wl, rank, world_size)

@@ -1,7 +1,7 @@
 // TEST INFRASTRUCTURE ONLY — never linked into, imported by or executed from the product path.
 //
 // Headless C-ABI harness around the GENUINE reference class, compiled from the sources where they
-// lie under /root/reference (see oracle/Makefile, target `ref`).  Nothing of the reference is copied
+// lie under $SPHSM_REFERENCE_DIR (see oracle/Makefile, target `ref`).  Nothing of the reference is copied
 // into this repo: this file only #includes the reference header and calls the reference's own
 // methods.  The resulting oracle/_ref/libsphsm_ref.so is (a) the pin for the C restatement in
 // oracle/sphsm_oracle.c (bit-identical on every fixture, tests/test_oracle_vs_ref.py), (b) the

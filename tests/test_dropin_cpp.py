@@ -1,8 +1,9 @@
 """The C++ drop-in class (include/dropin/SPH_SM_monodomain.h + libsphsm_dropin.so) behind the reference's main.cpp.
 
 CPU part: the headers keep the reference's source-level API (the UNMODIFIED reference main.cpp compiles against them and
-every SPH_SM_monodomain:: symbol it references is exported by libsphsm_dropin.so; where /root/reference is absent an
-in-repo translation unit that makes the same calls stands in), and the Particle layout is the reference's 132 bytes.
+every SPH_SM_monodomain:: symbol it references is exported by libsphsm_dropin.so; an in-repo translation unit that makes the
+same calls is always checked, main.cpp itself as well where $SPHSM_REFERENCE_DIR names a checkout of the reference), and the
+Particle layout is the reference's 132 bytes.
 GPU part: the headless replay of main.cpp's run protocol (sphsm_headless) against the oracle driven the same way.
 """
 import os
@@ -17,7 +18,7 @@ from sph_sm_monodomain_b200 import build
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 INC = os.path.join(ROOT, "include", "dropin")
 STUBS = os.path.join(ROOT, "tests", "stubs")
-REF_MAIN = "/root/reference/main.cpp"
+REF_MAIN = os.path.join(os.environ["SPHSM_REFERENCE_DIR"], "main.cpp") if os.environ.get("SPHSM_REFERENCE_DIR") else None
 
 # every call main.cpp (and the survey's boundary list, SURVEY.md §8b) makes on the class, as a stand-alone unit
 API_USER = r"""
@@ -90,7 +91,7 @@ def test_dropin_library_exports_what_main_cpp_links_against(tmp_path):
     user = tmp_path / "api_user.cpp"
     user.write_text(API_USER)
     units.append((str(user), []))
-    if os.path.exists(REF_MAIN):  # this container only: the genuine, unmodified viewer source (GL calls stubbed as declarations)
+    if REF_MAIN and os.path.exists(REF_MAIN):  # the genuine, unmodified viewer source (GL calls stubbed as declarations)
         units.append((REF_MAIN, ["-I", STUBS]))
     for k, (src, extra) in enumerate(units):
         obj = str(tmp_path / f"unit{k}.o")

@@ -1,10 +1,10 @@
 #!/usr/bin/env python
 """Generate tests/golden/*.npz from the GENUINE reference (oracle/_ref/libsphsm_ref.so, built by
-`make -C oracle ref` from /root/reference, g++ -O2 -ffp-contract=off).
+`make -C oracle ref` from $SPHSM_REFERENCE_DIR, g++ -O2 -ffp-contract=off).
 
 The reference has no tests or golden vectors of its own (SURVEY.md §4), so these files — outputs of the
 unmodified reference class on its own inputs — are the committed pin for the C restatement (oracle/) and
-the CUDA path.  Runs only where /root/reference exists (this container); the fixtures travel via git.
+the CUDA path.  Runs only where $SPHSM_REFERENCE_DIR names a checkout of the reference; the fixtures travel via git.
 
     python tools/make_golden.py            # ~2.5 min
 """
@@ -18,7 +18,10 @@ sys.path.insert(0, ROOT)
 from oracle import CpuSim  # noqa: E402
 from sph_sm_monodomain_b200 import inputs  # noqa: E402
 
-RES = "/root/reference/Resources/"
+REF_DIR = os.environ.get("SPHSM_REFERENCE_DIR")
+if not REF_DIR or not os.path.isdir(os.path.join(REF_DIR, "Resources")):
+    sys.exit("set SPHSM_REFERENCE_DIR to a checkout of the reference (this tool reads its Resources/*.csv)")
+RES = os.path.join(REF_DIR, "Resources", "")
 OUT = os.path.join(ROOT, "tests", "golden")
 
 STATE = ("pos", "vel", "dens", "pres", "Vm", "Inter_Vm", "Iion", "w", "stim")
