@@ -251,6 +251,46 @@ int sphsm_download_owned(sphsm_handle *h, int *ids, float *xyz, int cap, int *co
 int sphsm_comm_init_local(sphsm_handle **handles, int nranks);
 int sphsm_step_group(sphsm_handle **handles, int nranks, int nsteps);
 
+/* ---- recorder of the membrane-potential wave (no reference counterpart) ------------------------------------------------
+ * Activation / recovery time maps and probe traces ("virtual electrodes") of Vm, kept on the device by one small kernel at the
+ * end of every step, so that watching the wave costs a few bytes per particle per step instead of a download of every particle.
+ *
+ * Recording is off by default; while it is off nothing is allocated and the step launches nothing extra.  While it is on, every
+ * step that advances total_time_steps records that step, on every step path (fused, CUDA-graph replay, strict, staged with stage
+ * timing, sphsm_profile_step, the NCCL slab step, sphsm_step_group); a stand-alone sphsm_stage(1..9) records nothing.  The step
+ * index is total_time_steps after the step (the first step of a fresh handle is step 1).
+ *
+ * For each particle the step integrates, pre = the Vm the step started from (after any call made between steps, e.g. turnOffStim
+ * zeroing Vm) and post = the Vm the step produced:
+ *   upstroke    pre <  vm_up   && post >= vm_up    first_up = step if unset, last_up = step, n_up += 1
+ *   downstroke  pre >= vm_down && post <  vm_down  last_down = step
+ * A change of Vm made between steps (turnOffStim, uploads, set_masks) is not a crossing.  The rule has no state: in slab mode each
+ * crossing is seen by exactly one rank (the one that integrated the particle in that step), and per-rank maps merge exactly:
+ * first_up by minimum over set values, last_up / last_down by maximum, n_up by sum (sph_sm_monodomain_b200.slabs.merge_activation).
+ *
+ * Probes: up to SPHSM_RECORD_MAX_PROBES distinct original particle ids in [0, particle count) (the global count in slab mode),
+ * fixed when recording starts.  At every recorded step each rank stores (pos.xyz, Vm) after the step for the probes it integrated,
+ * in a ring of trace_rows rows (trace_rows * n_probes <= SPHSM_RECORD_MAX_TRACE_ENTRIES).  Each entry has an owned flag set only by
+ * the rank that wrote it, so ranks merge exactly (slabs.merge_traces).  Recording never pauses while it is on: the rows held are
+ * the last min(trace_rows, steps recorded) consecutive steps.
+ *
+ * Lifetime: sphsm_record_start (re)configures and clears; sphsm_record_stop and sphsm_destroy free the buffers; sphsm_record_reset
+ * clears the data and keeps the configuration; sphsm_load_state clears the data too (numbering continues at the snapshot's step
+ * counter + 1).  In slab mode every rank issues the recorder calls alike, like the state mutators; none of them is collective.
+ * Errors: SPHSM_ERR_INVALID for reversed or non-finite thresholds, duplicate or out-of-range probe ids, trace_rows <= 0 with
+ * probes, a size over the bounds below, and for reading or resetting while recording is off. */
+#define SPHSM_RECORD_MAX_PROBES 65536
+#define SPHSM_RECORD_MAX_TRACE_ENTRIES (1 << 24)
+int sphsm_record_start(sphsm_handle *h, float vm_up, float vm_down, const int *probe_ids, int n_probes, int trace_rows);
+int sphsm_record_stop(sphsm_handle *h);
+int sphsm_record_reset(sphsm_handle *h);
+/* The maps in original particle order, n entries each (n <= capacity; the particle count, global in slab mode); unset steps
+ * are -1.  A null array is skipped.  Synchronises. */
+int sphsm_get_activation(sphsm_handle *h, int *first_up, int *last_up, int *last_down, int *n_up, int n);
+/* Up to max_rows of the most recent trace rows, oldest first: *rows rows starting at step *first_step; xyzv[rows * n_probes * 4]
+ * = (pos.xyz, Vm) in probe order, owned[rows * n_probes] = 1 where this rank wrote the entry (0: entry zeroed).  Synchronises. */
+int sphsm_get_probe_trace(sphsm_handle *h, int max_rows, int *rows, int *first_step, float *xyzv, uint8_t *owned);
+
 /* Process-wide kernel-path switches for tests and tuning (no reference counterpart): "pass" = 6 (block-staged neighbour
  * passes, the default) | 4 (the gathered passes they are bit-identical to); "stage6" = 1 | 0 (0: every block of the
  * generation-6 kernels takes its in-kernel gathered path); "t6" = 128 | 64 targets per block; "b_step6" = 2 | 4 candidates

@@ -87,6 +87,11 @@ SYMBOLS = {
     "sphsm_download_owned": (C.c_int, [_H, _IP, _FP, C.c_int, _IP]),
     "sphsm_comm_init_local": (C.c_int, [C.POINTER(_H), C.c_int]),
     "sphsm_step_group": (C.c_int, [C.POINTER(_H), C.c_int, C.c_int]),
+    "sphsm_record_start": (C.c_int, [_H, C.c_float, C.c_float, _IP, C.c_int, C.c_int]),
+    "sphsm_record_stop": (C.c_int, [_H]),
+    "sphsm_record_reset": (C.c_int, [_H]),
+    "sphsm_get_activation": (C.c_int, [_H, _IP, _IP, _IP, _IP, C.c_int]),
+    "sphsm_get_probe_trace": (C.c_int, [_H, C.c_int, _IP, _IP, _FP, _U8P]),
     "sphsm_tune": (C.c_int, [C.c_char_p, C.c_int]),
     "sphsm_last_error": (C.c_char_p, [_H]),
 }

@@ -21,6 +21,7 @@
 #include "sphsm_pass4.cuh"
 #include "sphsm_pass4w.cuh"
 #include "sphsm_pass6.cuh"
+#include "sphsm_record.cuh"
 #include "sphsm_sm.cuh"
 #include "sphsm_sort.cuh"
 #include "sphsm_types.cuh"
@@ -175,6 +176,19 @@ struct sphsm_handle {
     int mom_n = 0;            // slab step: extent of the PRE-reorder arrays (old slots + both message regions) the REST-state sums scan
     int mom_begin = 0, mom_end = 0;  // slab step: the slots this rank integrated last step; its share of the per-step moment sums
     struct GroupTimer *gt = nullptr;
+    // activation maps / probe traces of Vm (sphsm_record.cuh, sphsm_host_record.cuh): nothing allocated or launched while off
+    struct Recorder {
+        bool on = false;
+        float vm_up = 0.f, vm_down = 0.f;
+        int cap = 0, n_probes = 0, rows = 0;
+        int *maps = nullptr;      // 4 x cap: first_up, last_up, last_down, n_up (by original id)
+        int *probe_of = nullptr;  // cap entries, -1 = not a probe
+        float4 *trace = nullptr;  // rows x n_probes ring
+        int *stamp = nullptr;     // rows x n_probes: step that wrote the entry
+        unsigned *ctl = nullptr;  // [0] step counter, [1] ticket
+        int dev_steps = 0;        // what ctl[0] holds once the queued steps have run
+        long long recorded = 0;   // steps recorded since start / reset
+    } rec;
 };
 
 #define CU(call)                                                                                   \
@@ -518,6 +532,7 @@ extern "C" int sphsm_destroy(sphsm_handle *h) {
     cudaFree(h->ghist); cudaFree(h->tile_state); cudaFree(h->tile_counter); cudaFree(h->cell_start); cudaFree(h->slot_of);
     cudaFree(h->d_dp); cudaFree(h->sm); cudaFree(h->partial); cudaFree(h->totals); cudaFree(h->scratch); cudaFree(h->d_aos); cudaFree(h->d_tmp);
     cudaFree(h->d_itmp);
+    cudaFree(h->rec.maps); cudaFree(h->rec.probe_of); cudaFree(h->rec.trace); cudaFree(h->rec.stamp); cudaFree(h->rec.ctl);
     for (int k = 0; k < 2; k++) { cudaFree(h->msg_send[k]); cudaFree(h->msg_recv[k]); }
     for (size_t k = 0; k < h->p2p_all.size(); k++)
         if (h->p2p_all[k] && h->p2p_all[k] != h->p2p_block) cudaIpcCloseMemHandle(h->p2p_all[k]);
@@ -1039,14 +1054,18 @@ extern "C" int sphsm_set_masks(sphsm_handle *h, const uint8_t *fixed, const floa
 }
 
 static void trace_mark(sphsm_handle *h, const char *label, bool side = false);  // SPHSM_TRACE (sphsm_host_slab.cuh)
-#include "sphsm_host_io.cuh"    // snapshot / restart, asynchronous per-frame I/O
-#include "sphsm_host_step.cuh"  // timers, neighbour grid, shape-matching sums, staged / fused step, graph replay
+static void record_clear(sphsm_handle *h);  // sphsm_host_record.cuh
+#include "sphsm_host_io.cuh"      // snapshot / restart, asynchronous per-frame I/O
+#include "sphsm_host_record.cuh"  // activation maps / probe traces: the per-step hook and the sphsm_record_* entry points
+#include "sphsm_host_step.cuh"    // timers, neighbour grid, shape-matching sums, staged / fused step, graph replay
 
 extern "C" int sphsm_step(sphsm_handle *h, int nsteps) {
     if (!h || nsteps < 0) return SPHSM_ERR_INVALID;
     CU(cudaSetDevice(h->prm.device));
     if (h->comm_mode == 2) return fail(h, SPHSM_ERR_COMM, "a local group steps through sphsm_step_group");
     if (h->failed) return fail(h, SPHSM_ERR_COMM, "the slab group stopped after a step error; re-upload the particle set and apply the slab again");
+    int rc0 = record_sync(h);
+    if (rc0) return rc0;
     CU(cudaEventRecord(h->ev_step0, h->stream));
     if (h->comm_mode == 1) {
         for (int s = 0; s < nsteps; s++) {
@@ -1113,8 +1132,9 @@ extern "C" int sphsm_profile_step(sphsm_handle *h, int nsteps, float out_ms[SPHS
     if (!h || !out_ms || nsteps <= 0) return SPHSM_ERR_INVALID;
     CU(cudaSetDevice(h->prm.device));
     for (int g = 0; g < SPHSM_NUM_KERNEL_GROUPS; g++) { h->group_ms[g] = 0.f; h->group_launches[g] = 0; }
+    int rc = record_sync(h);
+    if (rc) return rc;
     h->profiling = true;
-    int rc = SPHSM_OK;
     for (int s = 0; s < nsteps && rc == SPHSM_OK; s++) {
         if (h->comm_mode == 1) { rc = mg_step_nccl(h); continue; }
         rc = h->prm.strict ? fused_step<true>(h) : fused_step<false>(h);

@@ -441,6 +441,10 @@ static int fused_step(sphsm_handle *h) {
     }
     std::swap(h->cur.P, h->alt.P);
     gt.end_group(KG_PASS_B);
+    if (h->rec.on) {  // pre-step Vm in PB.w, post-step Vm in E.x, new positions in cur.P
+        if ((rc = record_launch(h, nullptr, n)) != 0) return rc;
+        gt.end_group(KG_OTHER);
+    }
     CU(cudaGetLastError());
     gt.finish();
     h->grid_valid = false;
@@ -466,7 +470,7 @@ static int timed_staged_step(sphsm_handle *h) {
         h->stage_time[st - 1] += ms * 1e-3;
     }
     h->inter_live = false;
-    return SPHSM_OK;
+    return record_launch(h, nullptr, h->n);  // (outside the stage timers; PB.w is stage 6's pre-step Vm, E.x stage 7's result)
 }
 
 static int mg_step_nccl(sphsm_handle *h);  // the slab step (below)
@@ -494,6 +498,12 @@ static std::string step_signature(const sphsm_handle *h) {
     const void *ptrs[] = {h->cell_start, h->cell_count, h->scan_state, h->scan_ctl, h->keys[0], h->keys[1], h->vals[0], h->vals[1], h->big_cells, h->big_count,
                           h->sm, h->partial, h->totals, h->d_dp, h->ghist, h->tile_state, h->tile_counter, h->scratch, h->skeys};
     put(ptrs, sizeof(ptrs));
+    const void *rec_ptrs[] = {h->rec.maps, h->rec.probe_of, h->rec.trace, h->rec.stamp, h->rec.ctl};  // (all null while recording is off)
+    put(rec_ptrs, sizeof(rec_ptrs));
+    const float rec_vm[] = {h->rec.vm_up, h->rec.vm_down};
+    put(rec_vm, sizeof(rec_vm));
+    const int rec_cfg[] = {(int)h->rec.on, h->rec.cap, h->rec.n_probes, h->rec.rows};
+    put(rec_cfg, sizeof(rec_cfg));
     const int flags[] = {h->counts_ready, h->bounds_ready, h->sorted_buf, g_pass_gen, h->red_blocks, h->sort_passes, (int)h->grid_valid, (int)warp_path(h), g_stage6, g_t6, g_b_step6};
     put(flags, sizeof(flags));
     return sig;

@@ -10,7 +10,7 @@ import ctypes as C
 
 import numpy as np
 
-from . import _capi
+from . import _capi, slabs
 from ._capi import Params, SphsmError  # noqa: F401
 
 # the reference's Particle layout (Particle.h:7-35), 132 bytes
@@ -283,6 +283,8 @@ class Sim:
         self._ck(self.lib.sphsm_comm_init(self.h, int(nranks), int(rank), buf))
 
     def set_slab(self, lo, hi):
+        if not self.comm_info()["slab_on"]:
+            self._n_global = self.n  # (every rank holds the whole set until its first slab is applied; ids stay global)
         self._ck(self.lib.sphsm_comm_set_slab(self.h, int(lo), int(hi)))
 
     def comm_info(self):
@@ -314,6 +316,43 @@ class Sim:
         cnt = C.c_int()
         self._ck(self.lib.sphsm_download_owned(self.h, _ip(ids), _fp(xyz), cap, C.byref(cnt)))
         return ids[: cnt.value].copy(), xyz[: cnt.value].copy()
+
+    # ---- recorder of the Vm wave (include/sphsm_b200.h: sphsm_record_*) ------------------------------------------------
+    def record_start(self, vm_up, vm_down=None, probes=None, trace_rows=0):
+        """Record activation / recovery times (Vm rising through vm_up, falling through vm_down; vm_down defaults to vm_up) of
+        every particle and, for the original ids in `probes`, (pos, Vm) after every step in a ring of `trace_rows` rows."""
+        ids = np.ascontiguousarray(np.asarray([] if probes is None else probes, dtype=np.int32).ravel())
+        down = vm_up if vm_down is None else vm_down
+        self._ck(self.lib.sphsm_record_start(self.h, float(vm_up), float(down), _ip(ids) if len(ids) else None, len(ids), int(trace_rows)))
+        self._probes, self._trace_rows = ids.copy(), int(trace_rows)
+
+    def record_stop(self):
+        self._ck(self.lib.sphsm_record_stop(self.h))
+
+    def record_reset(self):
+        self._ck(self.lib.sphsm_record_reset(self.h))
+
+    def activation(self, n=None):
+        """{"first_up", "last_up", "last_down", "n_up"}: int32 arrays by original id (n = the particle count, global in slab mode);
+        steps never seen are -1."""
+        if n is None:
+            n = self._n_global if self.comm_info()["slab_on"] else self.n
+        out = {k: np.zeros(n, np.int32) for k in ("first_up", "last_up", "last_down", "n_up")}
+        self._ck(self.lib.sphsm_get_activation(self.h, _ip(out["first_up"]), _ip(out["last_up"]), _ip(out["last_down"]),
+                                               _ip(out["n_up"]), int(n)))
+        return out
+
+    def probe_trace(self):
+        """(first_step, xyzv (rows, K, 4) float32 = (pos.xyz, Vm) after each step, owned (rows, K) bool), oldest row first."""
+        k = len(getattr(self, "_probes", ()))
+        cap = self._trace_rows if k else 0
+        rows, first = C.c_int(), C.c_int()
+        xyzv = np.zeros((max(cap, 1), max(k, 1), 4), np.float32)
+        owned = np.zeros((max(cap, 1), max(k, 1)), np.uint8)
+        self._ck(self.lib.sphsm_get_probe_trace(self.h, cap, C.byref(rows), C.byref(first), _fp(xyzv),
+                                                owned.ctypes.data_as(C.POINTER(C.c_uint8))))
+        r = rows.value
+        return first.value, xyzv[:r, :k].copy(), owned[:r, :k].astype(bool)
 
     # ---- timers / counters --------------------------------------------------------------------------------
     def enable_stage_timing(self, on=True):
@@ -369,6 +408,14 @@ class LocalGroup:
         if rc:
             msgs = [self.lib.sphsm_last_error(s.h).decode() for s in self.sims]
             raise SphsmError(f"sphsm_step_group failed ({rc}): {msgs}")
+
+    def activation(self, n_global):
+        """The recorder's activation maps of every virtual rank, merged (slabs.merge_activation)."""
+        return slabs.merge_activation(s.activation(n_global) for s in self.sims)
+
+    def probe_trace(self):
+        """The recorder's probe traces of every virtual rank, merged (slabs.merge_traces): (first_step, xyzv, owned)."""
+        return slabs.merge_traces(s.probe_trace() for s in self.sims)
 
     def gather_positions(self, n_global):
         """Owned particles of every virtual rank assembled by original id; also returns the owner rank per particle."""

@@ -1,6 +1,7 @@
 """Host-side slab decomposition for the multi-GPU path (SURVEY.md §8e): which axis to cut, the cell plane of a position
-(exactly as the device computes it), per-plane particle counts and the balanced partition into contiguous plane ranges.
-Pure numpy; the counts are combined across ranks by the caller (torch.distributed all_reduce in bench.py)."""
+(exactly as the device computes it), per-plane particle counts and the balanced partition into contiguous plane ranges, and the exact merge of the per-rank results of
+the Vm recorder (Sim.activation / Sim.probe_trace).  Pure numpy; per-rank values are combined by the caller (torch.distributed in
+bench.py and tools/record_mg.py, LocalGroup for virtual ranks)."""
 from __future__ import annotations
 
 import numpy as np
@@ -49,3 +50,44 @@ def partition_planes(hist: np.ndarray, nranks: int):
         cuts.append(c)
     cuts.append(nplanes)
     return [(cuts[k], cuts[k + 1]) for k in range(nranks)]
+
+
+ACTIVATION_KEYS = ("first_up", "last_up", "last_down", "n_up")
+
+
+def merge_activation(parts):
+    """Merge per-rank activation maps (dicts of int32 arrays by original id, as Sim.activation returns them).  Each crossing is
+    recorded by exactly one rank, so the merge is exact: first_up = minimum over the ranks that set it, last_up / last_down =
+    maximum, n_up = sum; a step no rank set stays -1."""
+    parts = list(parts)
+    if not parts:
+        raise ValueError("no parts to merge")
+    fu = np.stack([np.asarray(p["first_up"], np.int32) for p in parts])
+    big = np.iinfo(np.int32).max
+    first = np.where(fu >= 0, fu, big).min(axis=0)
+    out = {"first_up": np.where(first == big, -1, first).astype(np.int32)}
+    for k in ("last_up", "last_down"):
+        out[k] = np.stack([np.asarray(p[k], np.int32) for p in parts]).max(axis=0).astype(np.int32)
+    out["n_up"] = np.stack([np.asarray(p["n_up"], np.int32) for p in parts]).sum(axis=0, dtype=np.int64).astype(np.int32)
+    return out
+
+
+def merge_traces(parts):
+    """Merge per-rank probe traces (first_step, xyzv (rows, K, 4), owned (rows, K)) as Sim.probe_trace returns them: every entry
+    comes from the rank that integrated that probe in that step.  All parts must cover the same steps; an entry owned by two ranks
+    is an error.  Returns (first_step, xyzv, owned)."""
+    parts = list(parts)
+    if not parts:
+        raise ValueError("no parts to merge")
+    first = int(parts[0][0])
+    xyzv = np.zeros(np.shape(parts[0][1]), np.float32)
+    owned = np.zeros(xyzv.shape[:2], bool)
+    for f, x, o in parts:
+        x, o = np.asarray(x, np.float32), np.asarray(o, bool)
+        if int(f) != first or x.shape != xyzv.shape or o.shape != owned.shape:
+            raise ValueError("probe traces of different steps or shapes")
+        if (owned & o).any():
+            raise ValueError("a probe entry is owned by two ranks")
+        xyzv[o] = x[o]
+        owned |= o
+    return first, xyzv, owned
