@@ -291,6 +291,39 @@ int sphsm_get_activation(sphsm_handle *h, int *first_up, int *last_up, int *last
  * = (pos.xyz, Vm) in probe order, owned[rows * n_probes] = 1 where this rank wrote the entry (0: entry zeroed).  Synchronises. */
 int sphsm_get_probe_trace(sphsm_handle *h, int max_rows, int *rows, int *first_step, float *xyzv, uint8_t *owned);
 
+/* ---- extracellular electrograms at virtual electrodes (no reference counterpart) ----------------------------------------
+ * The extracellular potential a fixed electrode sees (a pseudo-ECG, or a surface EMG for the biceps model), summed over every
+ * particle on the device each step, so that it costs 20 bytes per particle per step instead of a download of every particle.
+ * For step s, each particle i the step integrated and each electrode e:
+ *   q_i      = vol_i * L_i        L_i = sum_j vol_j (Vm_j - Vm_i) B2(r_ij): the SPH Laplacian sum step s adds into Inter_Vm
+ *                                 (cpp:563), on the configuration and Vm the step started from; vol = mass / dens with the
+ *                                 density step s computed
+ *   phi_e(s) = gain * sum_i q_i / sqrt(|x_i - e|^2 + softening^2)
+ * x_i is the position the step started from.  This is the discrete pseudo-ECG integral (Plonsey; Gima & Rudy), phi =
+ * 1/(4 pi sigma_e) * integral of div(sigma_i grad Vm) / r dV, up to the caller's `gain`; no unit conversion is applied.  The
+ * softening length (> 0) keeps an electrode inside the tissue finite.  Electrodes stay fixed in space while the tissue moves.
+ *
+ * Off by default; while off nothing is allocated and the step launches nothing extra.  While on, every step path (as for the
+ * recorder above) ends with one extra launch and writes one row of n_electrodes doubles into a ring of `rows` rows; a
+ * stand-alone sphsm_stage(1..9) writes no row.  Rows are numbered like the recorder's steps (total_time_steps after the step),
+ * and with both on they number every step alike.  The electrograms are independent of the recorder: either can be on alone.
+ * On one device the values are bit-reproducible (fixed summation order, no atomics), graph replay or not.
+ *
+ * Lifetime: sphsm_egm_start (re)configures and clears; sphsm_egm_stop and sphsm_destroy free; sphsm_egm_reset clears the rows;
+ * sphsm_load_state clears them too (numbering continues at the snapshot's step counter + 1).  In slab mode each rank holds the
+ * partial sum over the particles it integrated (sum the ranks' rows, sph_sm_monodomain_b200.slabs.merge_electrograms); every
+ * rank issues the calls alike, and none of them is collective.
+ * Errors: SPHSM_ERR_INVALID for n_electrodes outside [1, SPHSM_EGM_MAX_ELECTRODES], non-finite coordinates or gain, a
+ * softening that is not positive and finite, rows <= 0 or rows * n_electrodes > SPHSM_RECORD_MAX_TRACE_ENTRIES, and for
+ * reading or resetting while off. */
+#define SPHSM_EGM_MAX_ELECTRODES 256
+/* xyz[3 * n_electrodes]: the electrodes' positions in world coordinates */
+int sphsm_egm_start(sphsm_handle *h, const float *xyz, int n_electrodes, float gain, float softening, int rows);
+int sphsm_egm_stop(sphsm_handle *h);
+int sphsm_egm_reset(sphsm_handle *h);
+/* up to max_rows of the most recent rows, oldest first: *rows rows from step *first_step; phi[rows * n_electrodes].  Synchronises. */
+int sphsm_get_egm(sphsm_handle *h, int max_rows, int *rows, int *first_step, double *phi);
+
 /* Process-wide kernel-path switches for tests and tuning (no reference counterpart): "pass" = 6 (block-staged neighbour
  * passes, the default) | 4 (the gathered passes they are bit-identical to); "stage6" = 1 | 0 (0: every block of the
  * generation-6 kernels takes its in-kernel gathered path); "t6" = 128 | 64 targets per block; "b_step6" = 2 | 4 candidates

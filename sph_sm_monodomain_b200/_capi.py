@@ -92,6 +92,10 @@ SYMBOLS = {
     "sphsm_record_reset": (C.c_int, [_H]),
     "sphsm_get_activation": (C.c_int, [_H, _IP, _IP, _IP, _IP, C.c_int]),
     "sphsm_get_probe_trace": (C.c_int, [_H, C.c_int, _IP, _IP, _FP, _U8P]),
+    "sphsm_egm_start": (C.c_int, [_H, _FP, C.c_int, C.c_float, C.c_float, C.c_int]),
+    "sphsm_egm_stop": (C.c_int, [_H]),
+    "sphsm_egm_reset": (C.c_int, [_H]),
+    "sphsm_get_egm": (C.c_int, [_H, C.c_int, _IP, _IP, _DP]),
     "sphsm_tune": (C.c_int, [C.c_char_p, C.c_int]),
     "sphsm_last_error": (C.c_char_p, [_H]),
 }

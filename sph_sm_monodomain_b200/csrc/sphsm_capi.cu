@@ -17,6 +17,7 @@
 #include <vector>
 
 #include "sphsm_comm.cuh"
+#include "sphsm_egm.cuh"
 #include "sphsm_pass.cuh"
 #include "sphsm_pass4.cuh"
 #include "sphsm_pass4w.cuh"
@@ -185,10 +186,22 @@ struct sphsm_handle {
         int *probe_of = nullptr;  // cap entries, -1 = not a probe
         float4 *trace = nullptr;  // rows x n_probes ring
         int *stamp = nullptr;     // rows x n_probes: step that wrote the entry
-        unsigned *ctl = nullptr;  // [0] step counter, [1] ticket
-        int dev_steps = 0;        // what ctl[0] holds once the queued steps have run
         long long recorded = 0;   // steps recorded since start / reset
     } rec;
+    // extracellular electrograms at virtual electrodes (sphsm_egm.cuh, sphsm_host_egm.cuh): nothing allocated or launched while off
+    struct Electrograms {
+        bool on = false;
+        int n_el = 0, rows = 0, grid = 0;  // grid: k_egm's blocks (fixed while on: the summation order depends on it)
+        float gain = 0.f, eps2 = 0.f;      // eps2 = softening^2
+        float *Q = nullptr;                // alloc_n + 8: pass B's source vol * L by slot (also cur.Q / alt.Q)
+        float4 *el = nullptr;              // n_el electrodes
+        double *partial = nullptr;         // grid x n_el
+        double *ring = nullptr;            // rows x n_el
+        long long recorded = 0;            // steps reduced since start / reset
+    } egm;
+    // the device step counter of the recorder and the electrograms (allocated while either is on; sphsm_host_record.cuh)
+    unsigned *step_ctl = nullptr;  // [0] total_time_steps before the step, [1] ticket of the kernel that advances it
+    int dev_steps = 0;             // what step_ctl[0] holds once the queued steps have run
 };
 
 #define CU(call)                                                                                   \
@@ -532,7 +545,8 @@ extern "C" int sphsm_destroy(sphsm_handle *h) {
     cudaFree(h->ghist); cudaFree(h->tile_state); cudaFree(h->tile_counter); cudaFree(h->cell_start); cudaFree(h->slot_of);
     cudaFree(h->d_dp); cudaFree(h->sm); cudaFree(h->partial); cudaFree(h->totals); cudaFree(h->scratch); cudaFree(h->d_aos); cudaFree(h->d_tmp);
     cudaFree(h->d_itmp);
-    cudaFree(h->rec.maps); cudaFree(h->rec.probe_of); cudaFree(h->rec.trace); cudaFree(h->rec.stamp); cudaFree(h->rec.ctl);
+    cudaFree(h->rec.maps); cudaFree(h->rec.probe_of); cudaFree(h->rec.trace); cudaFree(h->rec.stamp); cudaFree(h->step_ctl);
+    cudaFree(h->egm.Q); cudaFree(h->egm.el); cudaFree(h->egm.partial); cudaFree(h->egm.ring);
     for (int k = 0; k < 2; k++) { cudaFree(h->msg_send[k]); cudaFree(h->msg_recv[k]); }
     for (size_t k = 0; k < h->p2p_all.size(); k++)
         if (h->p2p_all[k] && h->p2p_all[k] != h->p2p_block) cudaIpcCloseMemHandle(h->p2p_all[k]);
@@ -1055,8 +1069,10 @@ extern "C" int sphsm_set_masks(sphsm_handle *h, const uint8_t *fixed, const floa
 
 static void trace_mark(sphsm_handle *h, const char *label, bool side = false);  // SPHSM_TRACE (sphsm_host_slab.cuh)
 static void record_clear(sphsm_handle *h);  // sphsm_host_record.cuh
+static void egm_clear(sphsm_handle *h);     // sphsm_host_egm.cuh
 #include "sphsm_host_io.cuh"      // snapshot / restart, asynchronous per-frame I/O
-#include "sphsm_host_record.cuh"  // activation maps / probe traces: the per-step hook and the sphsm_record_* entry points
+#include "sphsm_host_record.cuh"  // activation maps / probe traces, the step counter and the per-step hook they share; sphsm_record_*
+#include "sphsm_host_egm.cuh"     // electrograms at virtual electrodes: sphsm_egm_* / sphsm_get_egm
 #include "sphsm_host_step.cuh"    // timers, neighbour grid, shape-matching sums, staged / fused step, graph replay
 
 extern "C" int sphsm_step(sphsm_handle *h, int nsteps) {
@@ -1064,7 +1080,7 @@ extern "C" int sphsm_step(sphsm_handle *h, int nsteps) {
     CU(cudaSetDevice(h->prm.device));
     if (h->comm_mode == 2) return fail(h, SPHSM_ERR_COMM, "a local group steps through sphsm_step_group");
     if (h->failed) return fail(h, SPHSM_ERR_COMM, "the slab group stopped after a step error; re-upload the particle set and apply the slab again");
-    int rc0 = record_sync(h);
+    int rc0 = observe_sync(h);
     if (rc0) return rc0;
     CU(cudaEventRecord(h->ev_step0, h->stream));
     if (h->comm_mode == 1) {
@@ -1132,7 +1148,7 @@ extern "C" int sphsm_profile_step(sphsm_handle *h, int nsteps, float out_ms[SPHS
     if (!h || !out_ms || nsteps <= 0) return SPHSM_ERR_INVALID;
     CU(cudaSetDevice(h->prm.device));
     for (int g = 0; g < SPHSM_NUM_KERNEL_GROUPS; g++) { h->group_ms[g] = 0.f; h->group_launches[g] = 0; }
-    int rc = record_sync(h);
+    int rc = observe_sync(h);
     if (rc) return rc;
     h->profiling = true;
     for (int s = 0; s < nsteps && rc == SPHSM_OK; s++) {

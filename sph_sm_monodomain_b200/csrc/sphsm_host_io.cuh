@@ -68,6 +68,7 @@ extern "C" int sphsm_load_state(sphsm_handle *h, const char *path) {
     }
     h->total_steps = hd.total_steps;
     record_clear(h);  // recorded data belongs to the replaced particle set; numbering continues at the snapshot's step + 1
+    egm_clear(h);
     return SPHSM_OK;
 }
 

@@ -1,6 +1,7 @@
-// sphsm_host_record.cuh — host side of the Vm recorder (sphsm_record.cuh): its per-step hook and the sphsm_record_* / sphsm_get_*
-// entry points.  Host code of libsphsm_b200.so, textually included by sphsm_capi.cu (one translation unit: the handle, the LAUNCH / CU
-// macros and the static helpers defined there are in scope).
+// sphsm_host_record.cuh — host side of the Vm recorder (sphsm_record.cuh): the sphsm_record_* / sphsm_get_* entry points, and
+// the per-step hook and device step counter it shares with the electrograms (sphsm_host_egm.cuh).  Host code of libsphsm_b200.so,
+// textually included by sphsm_capi.cu (one translation unit: the handle, the LAUNCH / CU macros and the static helpers defined
+// there are in scope).
 //
 // While recording is off nothing is allocated and the step launches nothing extra.  While it is on, every step path (fused,
 // graph replay, strict, staged with stage timing, sphsm_profile_step, the NCCL slab step, sphsm_step_group) ends with one k_record
@@ -8,11 +9,58 @@
 // (step_signature), so starting or stopping recording picks or captures a different graph.
 #pragma once
 
+// ---- the step counter and the per-step hook shared by the recorder and the electrograms -------------------------------------
+static bool observe_on(const sphsm_handle *h) { return h->rec.on || h->egm.on; }
+
+// the device step counter follows total_time_steps: set it again when the host counter moved outside an observed step
+// (sphsm_load_state, a step with no particles).  Called at the entry of every stepping call, never inside a graph capture.
+static int observe_sync(sphsm_handle *h) {
+    if (!observe_on(h) || h->dev_steps == h->total_steps) return SPHSM_OK;
+    const unsigned v[2] = {(unsigned)h->total_steps, 0u};
+    CU(cudaMemcpyAsync(h->step_ctl, v, sizeof v, cudaMemcpyHostToDevice, h->stream));
+    h->dev_steps = h->total_steps;
+    return SPHSM_OK;
+}
+
+// a start: the counter exists while either observer is on (called once the starting one is on)
+static int step_ctl_attach(sphsm_handle *h) {
+    if (!h->step_ctl) CU(cudaMalloc(&h->step_ctl, 2 * sizeof(unsigned)));
+    h->dev_steps = h->total_steps - 1;  // (forces the counter upload)
+    return observe_sync(h);
+}
+
+// a stop: the last observer to go frees the counter (called once the stopping one is off)
+static void step_ctl_detach(sphsm_handle *h) {
+    if (observe_on(h) || !h->step_ctl) return;
+    cudaStreamSynchronize(h->stream);  // (a queued step may still write it)
+    cudaFree(h->step_ctl);
+    h->step_ctl = nullptr;
+    h->dev_steps = 0;
+}
+
+static int record_launch(sphsm_handle *h, const int *rng, int count, bool advance);
+static int egm_launch(sphsm_handle *h, const int *rng, int count);  // sphsm_host_egm.cuh
+
+// the per-step hook: right after the kernel that integrated the step, over the slots it integrated
+// (rng == nullptr: h->dp's own range, count = its length; slab step: the device range rng_all, count = own_bound).
+// One launch per observer that is on; the last one advances the step counter, so both number the step alike.
+static int observe_launch(sphsm_handle *h, const int *rng, int count) {
+    if (!observe_on(h)) return SPHSM_OK;
+    int rc;
+    count = std::max(count, 0);
+    if (h->rec.on && (rc = record_launch(h, rng, count, !h->egm.on)) != 0) return rc;
+    if (h->egm.on && (rc = egm_launch(h, rng, count)) != 0) return rc;
+    h->dev_steps++;
+    return SPHSM_OK;
+}
+
+// ---- the recorder ---------------------------------------------------------------------------------------------------------
 static void record_free(sphsm_handle *h) {
     auto &r = h->rec;
-    if (r.maps || r.ctl) cudaStreamSynchronize(h->stream);  // (a queued step may still write them)
-    cudaFree(r.maps); cudaFree(r.probe_of); cudaFree(r.trace); cudaFree(r.stamp); cudaFree(r.ctl);
+    if (r.maps) cudaStreamSynchronize(h->stream);  // (a queued step may still write them)
+    cudaFree(r.maps); cudaFree(r.probe_of); cudaFree(r.trace); cudaFree(r.stamp);
     r = sphsm_handle::Recorder{};
+    step_ctl_detach(h);
 }
 
 // data cleared, configuration kept: steps unset (-1), n_up 0, no trace row owned
@@ -25,22 +73,9 @@ static void record_clear(sphsm_handle *h) {
     r.recorded = 0;
 }
 
-// the device step counter follows total_time_steps: set it again when the host counter moved outside a recorded step
-// (sphsm_load_state, a step with no particles).  Called at the entry of every stepping call, never inside a graph capture.
-static int record_sync(sphsm_handle *h) {
+// advance: this launch is the hook's last and advances the step counter
+static int record_launch(sphsm_handle *h, const int *rng, int count, bool advance) {
     auto &r = h->rec;
-    if (!r.on || r.dev_steps == h->total_steps) return SPHSM_OK;
-    const unsigned v[2] = {(unsigned)h->total_steps, 0u};
-    CU(cudaMemcpyAsync(r.ctl, v, sizeof v, cudaMemcpyHostToDevice, h->stream));
-    r.dev_steps = h->total_steps;
-    return SPHSM_OK;
-}
-
-// the per-step hook: right after the kernel that integrated the step, over the slots it integrated
-// (rng == nullptr: h->dp's own range, count = its length; slab step: the device range rng_all, count = own_bound)
-static int record_launch(sphsm_handle *h, const int *rng, int count) {
-    auto &r = h->rec;
-    if (!r.on) return SPHSM_OK;
     RecArgs a;
     a.first_up = r.maps;
     a.last_up = r.maps + (size_t)r.cap;
@@ -53,11 +88,10 @@ static int record_launch(sphsm_handle *h, const int *rng, int count) {
     a.rows = std::max(r.rows, 1);
     a.vm_up = r.vm_up;
     a.vm_down = r.vm_down;
-    a.ctl = r.ctl;
-    count = std::max(count, 0);
+    a.ctl = h->step_ctl;
+    a.advance = advance ? 1 : 0;
     LAUNCH(k_record, std::max(1, cdiv(count, REC_THREADS)), REC_THREADS, h->dp, rng, count, (const int *)h->cur.ID, (const float4 *)h->cur.PB,
            (const float4 *)h->cur.E, (const float4 *)h->cur.P, a);
-    r.dev_steps++;
     r.recorded++;
     return SPHSM_OK;
 }
@@ -90,7 +124,6 @@ extern "C" int sphsm_record_start(sphsm_handle *h, float vm_up, float vm_down, c
     r.rows = n_probes > 0 ? trace_rows : 0;
     int rc = [&]() -> int {
         CU(cudaMalloc(&r.maps, (size_t)4 * r.cap * sizeof(int)));
-        CU(cudaMalloc(&r.ctl, 2 * sizeof(unsigned)));
         if (n_probes > 0) {
             CU(cudaMalloc(&r.probe_of, (size_t)r.cap * sizeof(int)));
             CU(cudaMalloc(&r.trace, (size_t)r.rows * n_probes * sizeof(float4)));
@@ -104,8 +137,7 @@ extern "C" int sphsm_record_start(sphsm_handle *h, float vm_up, float vm_down, c
         }
         r.on = true;
         record_clear(h);
-        r.dev_steps = h->total_steps - 1;  // (forces the counter upload)
-        int rc3 = record_sync(h);
+        int rc3 = step_ctl_attach(h);
         if (rc3) return rc3;
         CU(cudaGetLastError());
         CU(cudaStreamSynchronize(h->stream));
@@ -155,7 +187,7 @@ extern "C" int sphsm_get_probe_trace(sphsm_handle *h, int max_rows, int *rows, i
     const int K = r.n_probes;
     const int held = K > 0 ? (int)std::min<long long>(std::min<long long>(r.rows, r.recorded), max_rows) : 0;
     if (held > 0 && (!xyzv || !owned)) return fail(h, SPHSM_ERR_INVALID, "null output array");
-    const int last = r.dev_steps, first = last - held + 1;  // the last `held` steps, oldest first
+    const int last = h->dev_steps, first = last - held + 1;  // the last `held` steps, oldest first
     *rows = held;
     *first_step = held > 0 ? first : last + 1;
     if (held == 0) return SPHSM_OK;

@@ -706,8 +706,8 @@ static int mg_phase(sphsm_handle *h, int phase, int *coll, int *count) {
             }
             std::swap(h->cur.P, h->alt.P);
             if (h->gt) h->gt->end_group(KG_PASS_B);
-            if (h->rec.on) {  // over the owned slots this step integrated (both streams have joined)
-                if ((rc = record_launch(h, h->d_meta[h->meta_cur]->rng_all, h->own_bound)) != 0) return rc;
+            if (observe_on(h)) {  // over the owned slots this step integrated (both streams have joined)
+                if ((rc = observe_launch(h, h->d_meta[h->meta_cur]->rng_all, h->own_bound)) != 0) return rc;
                 if (h->gt) h->gt->end_group(KG_OTHER);
             }
             if (h->gt) {
@@ -838,7 +838,7 @@ extern "C" int sphsm_step_group(sphsm_handle **hs, int nranks, int nsteps) {
         sphsm_handle *h = hs[r];
         if (!h || h->comm_mode != 2 || h->nranks != nranks || h->rank != r) return fail(h, SPHSM_ERR_COMM, "not the local group made by sphsm_comm_init_local");
         int rc = mg_check(h);
-        if (!rc) rc = record_sync(h);
+        if (!rc) rc = observe_sync(h);
         if (rc) return rc;
     }
     sphsm_handle *h = hs[0];

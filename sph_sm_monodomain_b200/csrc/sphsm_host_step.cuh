@@ -276,7 +276,8 @@ static int run_stage(sphsm_handle *h, int stage) {
             break;
         case SPHSM_STAGE_FORCE:
             LAUNCH(k_refresh_derived, cdiv(n, 256), 256, n, h->cur, 0, 1);
-            LAUNCH((k_pass_b<STRICT, PB_FORCE_ONLY>), cdiv(n, 128), 128, h->dp, h->cur, (float4 *)nullptr, h->cell_start);
+            if (h->egm.on) LAUNCH((k_pass_b<STRICT, PB_FORCE_ONLY | PB_EGM>), cdiv(n, 128), 128, h->dp, h->cur, (float4 *)nullptr, h->cell_start);
+            else LAUNCH((k_pass_b<STRICT, PB_FORCE_ONLY>), cdiv(n, 128), 128, h->dp, h->cur, (float4 *)nullptr, h->cell_start);
             break;
         case SPHSM_STAGE_UPDATE:
             drop_counts(h);
@@ -355,10 +356,24 @@ static int launch_pass_a(sphsm_handle *h, int begin, int end, int hole_b = 0, in
     else LAUNCH6(k_pass_a6<128>, 128, false, g6_128, d, h->d_dp, h->cur, h->cell_start, h->key_sorted, g_stage6, rng);
     return SPHSM_OK;
 }
-template <int T, int STEP>
-static int launch_pass_b6(sphsm_handle *h, const DevParams &d, int grid, bool diag, uint32_t *nk, uint32_t *nr, uint32_t *ncnt, const int *rng) {
-    if (diag) LAUNCH6((k_pass_b6<T, STEP, true>), T, true, grid, d, h->d_dp, h->cur, h->alt.P, h->cell_start, h->key_sorted, nk, nr, ncnt, g_stage6, rng);
-    else LAUNCH6((k_pass_b6<T, STEP, false>), T, true, grid, d, h->d_dp, h->cur, h->alt.P, h->cell_start, h->key_sorted, nk, nr, ncnt, g_stage6, rng);
+// DIAG: ACC for the diagnostics download; EGM: the electrogram source Q (while electrograms are on)
+template <bool DIAG, bool EGM>
+static int launch_pass_b_as(sphsm_handle *h, const DevParams &d, int begin, int end, int hole_b, int hole_e, int count, uint32_t *nk, uint32_t *nr,
+                            uint32_t *ncnt, const int *rng) {
+    if (warp_path(h)) {
+        LAUNCH((k_pass_b4w<DIAG, EGM>), cdiv((long long)count * 32, PTW), PTW, d, h->cur, h->alt.P, h->cell_start, nk, nr, ncnt, count, rng);
+    } else if (g_pass_gen == 4) {
+        if (rng) LAUNCH((k_pass_b4<DIAG, true, EGM>), cdiv(count, PT4), PT4, d, h->d_dp, h->cur, h->alt.P, h->cell_start, h->key_sorted, nk, nr, ncnt, rng);
+        else LAUNCH((k_pass_b4<DIAG, false, EGM>), cdiv(count, PT4), PT4, d, h->d_dp, h->cur, h->alt.P, h->cell_start, h->key_sorted, nk, nr, ncnt, rng);
+    } else if (g_t6 == 64) {
+        const int grid = rng ? cdiv(count, 64) + 2 : grid6(begin, end, hole_b, hole_e, 64);
+        if (g_b_step6 == 4) LAUNCH6((k_pass_b6<64, 4, DIAG, EGM>), 64, true, grid, d, h->d_dp, h->cur, h->alt.P, h->cell_start, h->key_sorted, nk, nr, ncnt, g_stage6, rng);
+        else LAUNCH6((k_pass_b6<64, 2, DIAG, EGM>), 64, true, grid, d, h->d_dp, h->cur, h->alt.P, h->cell_start, h->key_sorted, nk, nr, ncnt, g_stage6, rng);
+    } else {
+        const int grid = rng ? cdiv(count, 128) + 2 : grid6(begin, end, hole_b, hole_e, 128);
+        if (g_b_step6 == 4) LAUNCH6((k_pass_b6<128, 4, DIAG, EGM>), 128, true, grid, d, h->d_dp, h->cur, h->alt.P, h->cell_start, h->key_sorted, nk, nr, ncnt, g_stage6, rng);
+        else LAUNCH6((k_pass_b6<128, 2, DIAG, EGM>), 128, true, grid, d, h->d_dp, h->cur, h->alt.P, h->cell_start, h->key_sorted, nk, nr, ncnt, g_stage6, rng);
+    }
     return SPHSM_OK;
 }
 static int launch_pass_b(sphsm_handle *h, int begin, int end, bool diag, int hole_b = 0, int hole_e = 0, bool file_counts = false,
@@ -368,23 +383,11 @@ static int launch_pass_b(sphsm_handle *h, int begin, int end, bool diag, int hol
     if (count <= 0) return SPHSM_OK;
     DevParams d = h->dp;
     d.own_begin = begin; d.own_end = end; d.hole_begin = hole_b; d.hole_len = hole_e - hole_b;
-
-    if (warp_path(h)) {
-        if (diag) LAUNCH(k_pass_b4w<true>, cdiv((long long)count * 32, PTW), PTW, d, h->cur, h->alt.P, h->cell_start, nk, nr, ncnt, count, rng);
-        else LAUNCH(k_pass_b4w<false>, cdiv((long long)count * 32, PTW), PTW, d, h->cur, h->alt.P, h->cell_start, nk, nr, ncnt, count, rng);
-    } else if (g_pass_gen == 4) {
-        if (diag && rng) LAUNCH((k_pass_b4<true, true>), cdiv(count, PT4), PT4, d, h->d_dp, h->cur, h->alt.P, h->cell_start, h->key_sorted, nk, nr, ncnt, rng);
-        else if (diag) LAUNCH((k_pass_b4<true, false>), cdiv(count, PT4), PT4, d, h->d_dp, h->cur, h->alt.P, h->cell_start, h->key_sorted, nk, nr, ncnt, rng);
-        else if (rng) LAUNCH((k_pass_b4<false, true>), cdiv(count, PT4), PT4, d, h->d_dp, h->cur, h->alt.P, h->cell_start, h->key_sorted, nk, nr, ncnt, rng);
-        else LAUNCH((k_pass_b4<false, false>), cdiv(count, PT4), PT4, d, h->d_dp, h->cur, h->alt.P, h->cell_start, h->key_sorted, nk, nr, ncnt, rng);
-    } else if (g_t6 == 64) {
-        const int grid = rng ? cdiv(count, 64) + 2 : grid6(begin, end, hole_b, hole_e, 64);
-        return g_b_step6 == 4 ? launch_pass_b6<64, 4>(h, d, grid, diag, nk, nr, ncnt, rng) : launch_pass_b6<64, 2>(h, d, grid, diag, nk, nr, ncnt, rng);
-    } else {
-        const int grid = rng ? cdiv(count, 128) + 2 : grid6(begin, end, hole_b, hole_e, 128);
-        return g_b_step6 == 4 ? launch_pass_b6<128, 4>(h, d, grid, diag, nk, nr, ncnt, rng) : launch_pass_b6<128, 2>(h, d, grid, diag, nk, nr, ncnt, rng);
-    }
-    return SPHSM_OK;
+    if (h->egm.on)
+        return diag ? launch_pass_b_as<true, true>(h, d, begin, end, hole_b, hole_e, count, nk, nr, ncnt, rng)
+                    : launch_pass_b_as<false, true>(h, d, begin, end, hole_b, hole_e, count, nk, nr, ncnt, rng);
+    return diag ? launch_pass_b_as<true, false>(h, d, begin, end, hole_b, hole_e, count, nk, nr, ncnt, rng)
+                : launch_pass_b_as<false, false>(h, d, begin, end, hole_b, hole_e, count, nk, nr, ncnt, rng);
 }
 
 // one fused step: grid, shape matching, pass A, pass B
@@ -428,7 +431,9 @@ static int fused_step(sphsm_handle *h) {
     if (STRICT) {
         LAUNCH((k_pass_a<STRICT, true, true>), cdiv(n, 128), 128, h->dp, h->cur, h->cell_start);
         gt.end_group(KG_PASS_A);
-        if (diag) LAUNCH((k_pass_b<STRICT, PB_FUSED_DIAG>), cdiv(n, 128), 128, h->dp, h->cur, h->alt.P, h->cell_start);
+        if (diag && h->egm.on) LAUNCH((k_pass_b<STRICT, PB_FUSED_DIAG | PB_EGM>), cdiv(n, 128), 128, h->dp, h->cur, h->alt.P, h->cell_start);
+        else if (diag) LAUNCH((k_pass_b<STRICT, PB_FUSED_DIAG>), cdiv(n, 128), 128, h->dp, h->cur, h->alt.P, h->cell_start);
+        else if (h->egm.on) LAUNCH((k_pass_b<STRICT, PB_FUSED | PB_EGM>), cdiv(n, 128), 128, h->dp, h->cur, h->alt.P, h->cell_start);
         else LAUNCH((k_pass_b<STRICT, PB_FUSED>), cdiv(n, 128), 128, h->dp, h->cur, h->alt.P, h->cell_start);
     } else {
         if ((rc = launch_pass_a(h, 0, n)) != 0) return rc;  // single GPU: own range = [0, n)
@@ -441,8 +446,8 @@ static int fused_step(sphsm_handle *h) {
     }
     std::swap(h->cur.P, h->alt.P);
     gt.end_group(KG_PASS_B);
-    if (h->rec.on) {  // pre-step Vm in PB.w, post-step Vm in E.x, new positions in cur.P
-        if ((rc = record_launch(h, nullptr, n)) != 0) return rc;
+    if (observe_on(h)) {  // pre-step Vm in PB.w, post-step Vm in E.x, new positions in cur.P, the source in Q
+        if ((rc = observe_launch(h, nullptr, n)) != 0) return rc;
         gt.end_group(KG_OTHER);
     }
     CU(cudaGetLastError());
@@ -470,7 +475,7 @@ static int timed_staged_step(sphsm_handle *h) {
         h->stage_time[st - 1] += ms * 1e-3;
     }
     h->inter_live = false;
-    return record_launch(h, nullptr, h->n);  // (outside the stage timers; PB.w is stage 6's pre-step Vm, E.x stage 7's result)
+    return observe_launch(h, nullptr, h->n);  // (outside the stage timers; PB.w is stage 6's pre-step Vm, E.x stage 7's result, Q stage 6's)
 }
 
 static int mg_step_nccl(sphsm_handle *h);  // the slab step (below)
@@ -498,12 +503,18 @@ static std::string step_signature(const sphsm_handle *h) {
     const void *ptrs[] = {h->cell_start, h->cell_count, h->scan_state, h->scan_ctl, h->keys[0], h->keys[1], h->vals[0], h->vals[1], h->big_cells, h->big_count,
                           h->sm, h->partial, h->totals, h->d_dp, h->ghist, h->tile_state, h->tile_counter, h->scratch, h->skeys};
     put(ptrs, sizeof(ptrs));
-    const void *rec_ptrs[] = {h->rec.maps, h->rec.probe_of, h->rec.trace, h->rec.stamp, h->rec.ctl};  // (all null while recording is off)
+    const void *rec_ptrs[] = {h->rec.maps, h->rec.probe_of, h->rec.trace, h->rec.stamp, h->step_ctl};  // (all null while recording is off)
     put(rec_ptrs, sizeof(rec_ptrs));
     const float rec_vm[] = {h->rec.vm_up, h->rec.vm_down};
     put(rec_vm, sizeof(rec_vm));
     const int rec_cfg[] = {(int)h->rec.on, h->rec.cap, h->rec.n_probes, h->rec.rows};
     put(rec_cfg, sizeof(rec_cfg));
+    const void *egm_ptrs[] = {h->egm.Q, h->egm.el, h->egm.partial, h->egm.ring};  // (all null while electrograms are off; Q is in Arrays too)
+    put(egm_ptrs, sizeof(egm_ptrs));
+    const float egm_f[] = {h->egm.gain, h->egm.eps2};
+    put(egm_f, sizeof(egm_f));
+    const int egm_cfg[] = {(int)h->egm.on, h->egm.n_el, h->egm.rows, h->egm.grid};
+    put(egm_cfg, sizeof(egm_cfg));
     const int flags[] = {h->counts_ready, h->bounds_ready, h->sorted_buf, g_pass_gen, h->red_blocks, h->sort_passes, (int)h->grid_valid, (int)warp_path(h), g_stage6, g_t6, g_b_step6};
     put(flags, sizeof(flags));
     return sig;

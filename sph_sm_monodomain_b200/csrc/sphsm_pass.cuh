@@ -4,7 +4,8 @@
 //                                   one sweep over the 27-cell stencil
 //   k_pass_b<STRICT, MODE>          ionic cell model (cpp:575-593) + pressure/viscosity force + SPH Laplacian of Vm
 //                                   (cpp:515-573) + integration, Vm clamp and walls (cpp:598-651) in one sweep;
-//                                   MODE selects the staged variants (force only) used by sphsm_stage()
+//                                   MODE selects the staged variants (force only) used by sphsm_stage(); MODE | PB_EGM
+//                                   also stores the electrogram source vol * L (sphsm_egm.cuh)
 //   k_cell_model, k_update          the stand-alone per-particle stages for sphsm_stage()
 // v1 mapping: one thread per particle over the cell-sorted SoA arrays; neighbouring threads sit in the same or
 // adjacent cells, so their float4 gathers hit the same L1 lines.
@@ -119,11 +120,13 @@ __device__ __forceinline__ void integrate(const DevParams &p, bool fixed, float 
 constexpr int PB_FORCE_ONLY = 0;  // stage 6: writes ACC = (acc, Inter_Vm)
 constexpr int PB_FUSED = 1;       // stages 5+6+7 in one sweep: cell model, force, integration; new pos -> Pout
 constexpr int PB_FUSED_DIAG = 2;  // PB_FUSED + ACC for the diagnostics download
+constexpr int PB_EGM = 4;         // flag on any of the above: Q = vol * L for the electrograms
 
-template <bool STRICT, int MODE>
+template <bool STRICT, int MODE_EGM>
 __global__ void __launch_bounds__(128) k_pass_b(const __grid_constant__ DevParams p, Arrays a, float4 *__restrict__ Pout,
                                                 const int *__restrict__ cell_start) {
     using A = Ar<STRICT>;
+    constexpr int MODE = MODE_EGM & ~PB_EGM;
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= p.n) return;
     const float4 pi = a.P[i];
@@ -201,6 +204,7 @@ __global__ void __launch_bounds__(128) k_pass_b(const __grid_constant__ DevParam
     // cpp:571: Inter_Vm += (sigma/(Beta*Cm))*Inter_Vm - ((Iion - stim*dt/mass)/Cm)   (the += form, Q9)
     const float ivm = A::add(L, A::sub(A::mul(p.diff_coef, L), A::div(A::sub(e.y, A::div(A::mul(e.w, p.dt), pi.w)), p.Cm)));
     if (MODE == PB_FORCE_ONLY || MODE == PB_FUSED_DIAG) a.ACC[i] = make_float4(ax, ay, az, ivm);
+    if (MODE_EGM & PB_EGM) a.Q[i] = A::mul(vi.w, L);
     if (MODE != PB_FORCE_ONLY) {
         float4 v4 = a.VEL[i];
         const bool fixed = __float_as_int(a.O[i].w) != 0;

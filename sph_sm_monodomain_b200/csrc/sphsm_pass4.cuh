@@ -301,9 +301,10 @@ __device__ __forceinline__ void integrate_fast(const DevParams &p, bool fixed, f
 // pass B's per-particle tail, shared by the thread-per-particle and the warp-per-particle kernels: acceleration, Inter_Vm
 // (cpp:568-571), Update_Properties (cpp:602-649), and — when cell_count is given — the next step's counting-sort input.
 // e4 = (Vm, Iion, w, stim) AFTER the ionic model; L = the SPH Laplacian sum of Vm.
+// EGM: also stores the electrogram source vol * L (vi.w = m / dens_new) into a.Q (sphsm_egm.cuh).
 // dens = this particle's new density (S.y, written by pass A); the old velocity is not an input of the step's last stage
 // (cpp:605: vel = inter_vel + acc * dt / mass), so VEL is written here without having been read.
-template <bool DIAG>
+template <bool DIAG, bool EGM>
 __device__ __forceinline__ void pass_b_finish(const DevParams &p, const Arrays &a, float4 *__restrict__ Pout, const int i, const float4 pi,
                                               const float4 vi, float4 e4, const float dens, const bool fixed, float ax, float ay, float az,
                                               const float L, const float inv_mass, uint32_t *__restrict__ next_keys,
@@ -318,6 +319,7 @@ __device__ __forceinline__ void pass_b_finish(const DevParams &p, const Arrays &
     const float dtm = p.dt * inv_mass;
     const float ivm = SPHSM_FAST_ODE ? L + (p.diff_coef * L - (e4.y - e4.w * dtm) / p.Cm) : L + (p.diff_coef * L - (e4.y - div_rn_z(e4.w * p.dt, pi.w)) / p.Cm);
     if (DIAG) a.ACC[i] = make_float4(ax, ay, az, ivm);
+    if (EGM) a.Q[i] = vi.w * L;
     float x = pi.x, y = pi.y, z = pi.z;
     integrate_fast(p, fixed, dtm, vi.x, vi.y, vi.z, ax, ay, az, ivm, pi.w, x, y, z, v4.x, v4.y, v4.z, e4.x);
     Pout[i] = make_float4(x, y, z, pi.w);
@@ -338,7 +340,7 @@ __device__ __forceinline__ void pass_b_finish(const DevParams &p, const Arrays &
 // (reference cpp:575-593, 515-573, 598-651).  PB = (pos.xyz, Vm) is the neighbour record of this pass.
 // cell_count != nullptr: the thread also files its particle's NEW position for the next step's counting sort (key, provisional
 // rank in the cell, per-cell count — what k_cell_count does, without re-reading the positions)
-template <bool DIAG>
+template <bool DIAG, bool EGM>
 __device__ __forceinline__ void pass_b4_one(const DevParams &p, const DevParams *__restrict__ g, const Arrays &a, float4 *__restrict__ Pout,
                                             const int *__restrict__ cell_start, const uint32_t *__restrict__ skey, uint32_t *__restrict__ next_keys,
                                             uint32_t *__restrict__ next_rank, uint32_t *__restrict__ cell_count, const int i, const unsigned slist) {
@@ -438,9 +440,9 @@ __device__ __forceinline__ void pass_b4_one(const DevParams &p, const DevParams 
                 lo = lbase;
             });
     }
-    pass_b_finish<DIAG>(p, a, Pout, i, pi, vi, e4, si.y, fixed, ax, ay, az, L + L1, inv_mass, next_keys, next_rank, cell_count);
+    pass_b_finish<DIAG, EGM>(p, a, Pout, i, pi, vi, e4, si.y, fixed, ax, ay, az, L + L1, inv_mass, next_keys, next_rank, cell_count);
 }
-template <bool DIAG, bool RNG>
+template <bool DIAG, bool RNG, bool EGM>
 __global__ void __launch_bounds__(PT4, SPHSM_B_MINB) k_pass_b4(const __grid_constant__ DevParams p, const DevParams *__restrict__ g, Arrays a,
                                                 float4 *__restrict__ Pout, const int *__restrict__ cell_start, const uint32_t *__restrict__ skey,
                                                 uint32_t *__restrict__ next_keys, uint32_t *__restrict__ next_rank, uint32_t *__restrict__ cell_count,
@@ -457,7 +459,7 @@ __global__ void __launch_bounds__(PT4, SPHSM_B_MINB) k_pass_b4(const __grid_cons
         if (i >= p.hole_begin) i += p.hole_len;
         if (i >= p.own_end) return;
     }
-    pass_b4_one<DIAG>(p, g, a, Pout, cell_start, skey, next_keys, next_rank, cell_count, i, (unsigned)__cvta_generic_to_shared(s_list) + 4u * threadIdx.x);
+    pass_b4_one<DIAG, EGM>(p, g, a, Pout, cell_start, skey, next_keys, next_rank, cell_count, i, (unsigned)__cvta_generic_to_shared(s_list) + 4u * threadIdx.x);
 }
 
 }  // namespace sphsm

@@ -83,7 +83,7 @@ __global__ void __launch_bounds__(PTW) k_pass_a4w(const __grid_constant__ DevPar
 // ---------------------------------------------------------------------------------------------------
 // pass B: ionic cell model + pressure / viscosity force + SPH Laplacian of Vm + integration and walls
 // (reference cpp:575-593, 515-573, 598-651)
-template <bool DIAG>
+template <bool DIAG, bool EGM>
 __global__ void __launch_bounds__(PTW) k_pass_b4w(const __grid_constant__ DevParams p, Arrays a, float4 *__restrict__ Pout,
                                                   const int *__restrict__ cell_start, uint32_t *__restrict__ next_keys,
                                                   uint32_t *__restrict__ next_rank, uint32_t *__restrict__ cell_count, int count,
@@ -148,7 +148,7 @@ __global__ void __launch_bounds__(PTW) k_pass_b4w(const __grid_constant__ DevPar
     ay = warp_sum(ay);
     az = warp_sum(az);
     L = warp_sum(L);
-    if (lane == 0) pass_b_finish<DIAG>(p, a, Pout, i, pi, vi, e4, si.y, fixed, ax, ay, az, L, inv_mass, next_keys, next_rank, cell_count);
+    if (lane == 0) pass_b_finish<DIAG, EGM>(p, a, Pout, i, pi, vi, e4, si.y, fixed, ax, ay, az, L, inv_mass, next_keys, next_rank, cell_count);
 }
 
 }  // namespace sphsm

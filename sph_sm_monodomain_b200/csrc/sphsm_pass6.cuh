@@ -417,7 +417,7 @@ __device__ __forceinline__ void pass_b6_neighbours(const DevParams *__restrict__
 
 // cell_count != nullptr: the thread also files its particle's NEW position for the next step's counting sort (key, provisional
 // rank in the cell, per-cell count — what k_cell_count does, without re-reading the positions)
-template <int T, int STEP, bool DIAG>
+template <int T, int STEP, bool DIAG, bool EGM>
 __global__ void __launch_bounds__(T, 640 / T) k_pass_b6(const __grid_constant__ DevParams p, const DevParams *__restrict__ g, Arrays a,
                                                float4 *__restrict__ Pout, const int *__restrict__ cell_start, const uint32_t *__restrict__ skey,
                                                uint32_t *__restrict__ next_keys, uint32_t *__restrict__ next_rank, uint32_t *__restrict__ cell_count,
@@ -466,7 +466,7 @@ __global__ void __launch_bounds__(T, 640 / T) k_pass_b6(const __grid_constant__ 
     } else if (valid) {
         pass_b6_neighbours<L, T, STEP, false>(g, a, cell_start, key, smem0, 3, 0, pi, vi, Vm_i, si.x, ax, ay, az, Lsum);
     }
-    if (live) pass_b_finish<DIAG>(p, a, Pout, i, pi, vi, e4, si.y, fixed, ax, ay, az, Lsum, inv_mass, next_keys, next_rank, cell_count);
+    if (live) pass_b_finish<DIAG, EGM>(p, a, Pout, i, pi, vi, e4, si.y, fixed, ax, ay, az, Lsum, inv_mass, next_keys, next_rank, cell_count);
 }
 
 }  // namespace sphsm

@@ -20,7 +20,9 @@
 //
 // The step number comes from device memory, not from a kernel argument (a replayed CUDA graph reuses its captured arguments):
 // ctl[0] is total_time_steps before the step (set by the host when recording starts or the host counter changes outside a
-// step); the last block to finish (ticket in ctl[1]) advances it.  One launch per step.
+// step).  The counter is shared with the electrograms (sphsm_egm.cuh) and advanced once per step by the last kernel of the
+// step's hook: here (advance = 1) when electrograms are off, the last block to finish (ticket in ctl[1]) advancing it; k_egm
+// otherwise.  One launch per step.
 #pragma once
 #include "sphsm_pass4.cuh"
 #include "sphsm_types.cuh"
@@ -35,6 +37,7 @@ struct RecArgs {
     int n_probes, rows;
     float vm_up, vm_down;
     unsigned *ctl;                                // [0] steps recorded up to (= total_time_steps), [1] ticket
+    int advance;                                  // 1: this launch advances ctl[0] (0: k_egm follows and does)
 };
 
 constexpr int REC_THREADS = 256;
@@ -68,6 +71,7 @@ __global__ void __launch_bounds__(REC_THREADS) k_record(const __grid_constant__ 
         }
     }
     // last block out advances the step counter (every block has read it by then)
+    if (!r.advance) return;
     __shared__ bool last;
     __syncthreads();
     if (threadIdx.x == 0) {

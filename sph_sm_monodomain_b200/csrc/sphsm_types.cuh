@@ -12,6 +12,7 @@
 //   PB   float4  (pos.xyz, Vm)                     written by the reorder, gathered by pass B (fast path)
 //   VN   float   m/dens_new (= V.w), dense         written by pass A, gathered by pass B's phase 1 (fast path)
 //   ACC  float4  (acc.xyz, Inter_Vm)               staged / diagnostics mode only
+//   Q    float   vol * L, pass B's source strength  electrograms only (sphsm_egm.cuh); null while they are off
 //   GOAL float4  (goal.xyz, -)  PV float4 (predicted_vel.xyz, -)   diagnostics mode only
 //   COLD_GOAL / COLD_PV float4 by ORIGINAL index: the frozen mGoalPos / predicted_vel of fixed particles
 //        (the reference never updates them for mFixed particles, cpp:228,326,431)
@@ -64,6 +65,7 @@ struct Arrays {
     float *VN;   // m/dens_new again, as a DENSE float array: pass B's phase 1 reads it for every candidate, and a 4-byte
                  // gather from the 16-byte-strided V.w costs four L1 wavefronts per warp where this costs one
     float4 *COLD_GOAL, *COLD_PV;
+    float *Q;    // electrograms only: the same buffer in both ping-pong sets (written and read within one step)
 };
 
 // Shape-matching results shared between the solve and the per-particle goal kernel.

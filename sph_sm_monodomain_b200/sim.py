@@ -354,6 +354,29 @@ class Sim:
         r = rows.value
         return first.value, xyzv[:r, :k].copy(), owned[:r, :k].astype(bool)
 
+    # ---- electrograms at virtual electrodes (include/sphsm_b200.h: sphsm_egm_*) -------------------------------------
+    def egm_start(self, electrodes, gain=1.0, softening=None, rows=1024):
+        """Every step, phi_e = gain * sum_i vol_i L_i / sqrt(|x_i - e|^2 + softening^2) at each electrode e (an (E, 3) array of
+        fixed world positions, E <= 256), kept on the device in a ring of `rows` steps.  softening defaults to kernel_h."""
+        el = np.ascontiguousarray(np.asarray(electrodes, dtype=np.float32).reshape(-1, 3))
+        eps = self.get_params().kernel_h if softening is None else softening
+        self._ck(self.lib.sphsm_egm_start(self.h, _fp(el), len(el), float(gain), float(eps), int(rows)))
+        self._egm_shape = (int(rows), len(el))
+
+    def egm_stop(self):
+        self._ck(self.lib.sphsm_egm_stop(self.h))
+
+    def egm_reset(self):
+        self._ck(self.lib.sphsm_egm_reset(self.h))
+
+    def electrogram(self):
+        """(first_step, phi (rows, E) float64), oldest row first: the rows held, up to the ring's length."""
+        cap, e = getattr(self, "_egm_shape", (0, 1))
+        rows, first = C.c_int(), C.c_int()
+        phi = np.zeros((max(cap, 1), e), np.float64)
+        self._ck(self.lib.sphsm_get_egm(self.h, cap, C.byref(rows), C.byref(first), phi.ctypes.data_as(C.POINTER(C.c_double))))
+        return first.value, phi[: rows.value].copy()
+
     # ---- timers / counters --------------------------------------------------------------------------------
     def enable_stage_timing(self, on=True):
         self._ck(self.lib.sphsm_enable_stage_timing(self.h, int(on)))
@@ -416,6 +439,10 @@ class LocalGroup:
     def probe_trace(self):
         """The recorder's probe traces of every virtual rank, merged (slabs.merge_traces): (first_step, xyzv, owned)."""
         return slabs.merge_traces(s.probe_trace() for s in self.sims)
+
+    def electrogram(self):
+        """The electrograms of every virtual rank, summed in rank order (slabs.merge_electrograms): (first_step, phi)."""
+        return slabs.merge_electrograms(s.electrogram() for s in self.sims)
 
     def gather_positions(self, n_global):
         """Owned particles of every virtual rank assembled by original id; also returns the owner rank per particle."""

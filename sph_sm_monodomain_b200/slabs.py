@@ -1,6 +1,6 @@
 """Host-side slab decomposition for the multi-GPU path (SURVEY.md §8e): which axis to cut, the cell plane of a position
-(exactly as the device computes it), per-plane particle counts and the balanced partition into contiguous plane ranges, and the exact merge of the per-rank results of
-the Vm recorder (Sim.activation / Sim.probe_trace).  Pure numpy; per-rank values are combined by the caller (torch.distributed in
+(exactly as the device computes it), per-plane particle counts and the balanced partition into contiguous plane ranges, the exact merge of the per-rank results of
+the Vm recorder (Sim.activation / Sim.probe_trace) and the sum of the per-rank electrograms (Sim.electrogram).  Pure numpy; per-rank values are combined by the caller (torch.distributed in
 bench.py and tools/record_mg.py, LocalGroup for virtual ranks)."""
 from __future__ import annotations
 
@@ -91,3 +91,19 @@ def merge_traces(parts):
         xyzv[o] = x[o]
         owned |= o
     return first, xyzv, owned
+
+
+def merge_electrograms(parts):
+    """Sum per-rank electrograms (first_step, phi (rows, E)) as Sim.electrogram returns them, in rank order: each rank holds the
+    sum over the particles it integrated.  All parts must cover the same steps and electrodes.  Returns (first_step, phi)."""
+    parts = list(parts)
+    if not parts:
+        raise ValueError("no parts to merge")
+    first = int(parts[0][0])
+    phi = np.zeros(np.shape(parts[0][1]), np.float64)
+    for f, p in parts:
+        p = np.asarray(p, np.float64)
+        if int(f) != first or p.shape != phi.shape:
+            raise ValueError("electrograms of different steps or shapes")
+        phi += p
+    return first, phi
