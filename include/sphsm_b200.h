@@ -324,12 +324,12 @@ int sphsm_egm_reset(sphsm_handle *h);
 /* up to max_rows of the most recent rows, oldest first: *rows rows from step *first_step; phi[rows * n_electrodes].  Synchronises. */
 int sphsm_get_egm(sphsm_handle *h, int max_rows, int *rows, int *first_step, double *phi);
 
-/* Process-wide kernel-path switches for tests and tuning (no reference counterpart): "pass" = 6 (block-staged neighbour
- * passes, the default) | 4 (the gathered passes they are bit-identical to); "stage6" = 1 | 0 (0: every block of the
- * generation-6 kernels takes its in-kernel gathered path); "t6" = 128 | 64 targets per block; "b_step6" = 2 | 4 candidates
- * per iteration of the force pass; "warp_path" = 1 | 0 (0: small dense sets take the thread-per-particle kernels too).  The
- * same switches are read once from $SPHSM_PASS, $SPHSM_STAGE6, $SPHSM_T6, $SPHSM_B_STEP6, $SPHSM_WARP_PATH.  "pass", "stage6",
- * "t6" and "b_step6" change no result bit; "warp_path" changes the order of the floating-point sums. */
+/* Process-wide switches for tests and tuning (no reference counterpart); the first value is the default:
+ *   "warp_path"  = 1 | 0  0: small dense sets take the thread-per-particle neighbour passes too (changes the order of the
+ *                         floating-point sums);
+ *   "x1_dynamic" = 0 | 1  1: the ncclSend / ncclRecv messages of exchange 1 follow the face populations (sphsm_comm_x1_sizes;
+ *                         every rank alike).
+ * Both are read once from $SPHSM_WARP_PATH and $SPHSM_X1_DYNAMIC.  Any other name or value returns SPHSM_ERR_INVALID. */
 int sphsm_tune(const char *name, int value);
 
 const char *sphsm_last_error(sphsm_handle *h);

@@ -21,7 +21,6 @@
 #include "sphsm_pass.cuh"
 #include "sphsm_pass4.cuh"
 #include "sphsm_pass4w.cuh"
-#include "sphsm_pass6.cuh"
 #include "sphsm_record.cuh"
 #include "sphsm_sm.cuh"
 #include "sphsm_sort.cuh"
@@ -217,15 +216,6 @@ struct sphsm_handle {
 
 // SPHSM_SYNC_DEBUG=1 in the environment synchronises after every launch and names the kernel that faulted
 static const bool g_sync_debug = getenv("SPHSM_SYNC_DEBUG") != nullptr;
-// SPHSM_PASS selects the fast-path neighbour passes: 4 = the gathered thread-per-particle passes of sphsm_pass4.cuh (production),
-// 6 = sphsm_pass6.cuh (block-staged stencil spans: bit-identical, measured slower, kept as the documented experiment).
-// SPHSM_STAGE6=0 makes every block of the generation-6 kernels take their in-kernel gathered path; SPHSM_T6 = 64 | 128 targets per
-// block; SPHSM_B_STEP6 = 2 | 4 candidates per iteration of pass B's phase 1.
-// The same four switches can be changed at run time with sphsm_tune("pass" | "stage6" | "t6" | "b_step6", value) (tests).
-static int g_pass_gen = getenv("SPHSM_PASS") ? atoi(getenv("SPHSM_PASS")) : 4;
-static int g_stage6 = getenv("SPHSM_STAGE6") ? atoi(getenv("SPHSM_STAGE6")) : 1;
-static int g_t6 = getenv("SPHSM_T6") ? atoi(getenv("SPHSM_T6")) : 128;
-static int g_b_step6 = getenv("SPHSM_B_STEP6") ? atoi(getenv("SPHSM_B_STEP6")) : 2;
 // 1: ncclSend / ncclRecv exchange-1 messages sized from the lagged face populations; 0 (default): always the full halo capacity.
 // Process-wide: every rank of a group must run with the same setting (the two sides of a face derive the message size from it).
 // Off by default: a REGULAR lattice moves a whole lattice plane across a cell boundary in one step, which doubles a face
@@ -238,11 +228,7 @@ static int g_warp_path = getenv("SPHSM_WARP_PATH") ? atoi(getenv("SPHSM_WARP_PAT
 extern "C" int sphsm_tune(const char *name, int value) {
     if (!name) return SPHSM_ERR_INVALID;
     const std::string n(name);
-    if (n == "pass" && (value == 4 || value == 6)) g_pass_gen = value;
-    else if (n == "stage6" && (value == 0 || value == 1)) g_stage6 = value;
-    else if (n == "t6" && (value == 64 || value == 128)) g_t6 = value;
-    else if (n == "b_step6" && (value == 2 || value == 4)) g_b_step6 = value;
-    else if (n == "warp_path" && (value == 0 || value == 1)) g_warp_path = value;
+    if (n == "warp_path" && (value == 0 || value == 1)) g_warp_path = value;
     else if (n == "x1_dynamic" && (value == 0 || value == 1)) g_x1_dynamic = value;
     else return SPHSM_ERR_INVALID;
     return SPHSM_OK;

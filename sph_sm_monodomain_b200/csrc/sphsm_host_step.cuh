@@ -307,73 +307,27 @@ static bool warp_path(const sphsm_handle *h) {
     if (n > limit || h->host_cells.empty()) return false;
     return (double)n >= 3.0 * (double)h->host_cells.size();  // >= 3 particles per occupied cell: rows long enough for a warp
 }
-// slots [begin, end) minus the hole [hole_b, hole_e) (generation-4 kernels only)
-// blocks of a generation-6 launch: the two ranges on either side of the hole are cut into blocks separately (block_range6)
-static int grid6(int begin, int end, int hole_b, int hole_e, int T) {
-    if (hole_e > hole_b) return cdiv(hole_b - begin, T) + cdiv(end - hole_e, T);
-    return cdiv(end - begin, T);
-}
-template <class K>
-static int prepare6(sphsm_handle *h, K kern, unsigned bytes) {  // dynamic shared memory beyond 48 KB needs the opt-in; carve-out: all of it
-    static std::unordered_set<const void *> done;
-    if (done.count((const void *)kern)) return SPHSM_OK;
-    CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
-    CU(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    done.insert((const void *)kern);
-    return SPHSM_OK;
-}
-#define LAUNCH6(kern, T, WITH4, grid, ...)                                                                              \
-    do {                                                                                                                \
-        const unsigned bytes_ = Lay6<T, WITH4>::BYTES;                                                                  \
-        int rc_ = prepare6(h, kern, bytes_);                                                                            \
-        if (rc_) return rc_;                                                                                            \
-        if (!h->dry_run) kern<<<(grid), (T), bytes_, h->launch_stream>>>(__VA_ARGS__);                                   \
-        h->launches++;                                                                                                  \
-        if (g_sync_debug) {                                                                                             \
-            cudaError_t e_ = cudaStreamSynchronize(h->launch_stream);                                                   \
-            if (e_ != cudaSuccess) {                                                                                    \
-                h->err = std::string("kernel ") + #kern + " failed: " + cudaGetErrorString(e_);                         \
-                fprintf(stderr, "[sphsm] %s\n", h->err.c_str());                                                        \
-                return SPHSM_ERR_CUDA;                                                                                  \
-            }                                                                                                           \
-        }                                                                                                               \
-    } while (0)
 
 // slots [begin, end) minus the hole [hole_b, hole_e).  rng != nullptr (slab step): the range is read from device memory
 // ({begin, end, hole_begin, hole_len}) and [begin, end) / the hole only size the grid: `end - begin - hole` is an upper bound of the
-// target count, and with a hole the two sides may hold up to that many targets EACH (generation 6 cuts them into blocks separately).
+// target count.
 static int launch_pass_a(sphsm_handle *h, int begin, int end, int hole_b = 0, int hole_e = 0, const int *rng = nullptr) {
     const int count = end - begin - (hole_e - hole_b);
     if (count <= 0) return SPHSM_OK;
     DevParams d = h->dp;
     d.own_begin = begin; d.own_end = end; d.hole_begin = hole_b; d.hole_len = hole_e - hole_b;
 
-    const int g6_128 = rng ? cdiv(count, 128) + 2 : grid6(begin, end, hole_b, hole_e, 128), g6_64 = rng ? cdiv(count, 64) + 2 : grid6(begin, end, hole_b, hole_e, 64);
     if (warp_path(h)) LAUNCH(k_pass_a4w, cdiv((long long)count * 32, PTW), PTW, d, h->cur, h->cell_start, count, rng);
-    else if (g_pass_gen == 4 && rng) LAUNCH(k_pass_a4<true>, cdiv(count, PT4), PT4, d, h->d_dp, h->cur, h->cell_start, h->key_sorted, rng);
-    else if (g_pass_gen == 4) LAUNCH(k_pass_a4<false>, cdiv(count, PT4), PT4, d, h->d_dp, h->cur, h->cell_start, h->key_sorted, rng);
-    else if (g_t6 == 64) LAUNCH6(k_pass_a6<64>, 64, false, g6_64, d, h->d_dp, h->cur, h->cell_start, h->key_sorted, g_stage6, rng);
-    else LAUNCH6(k_pass_a6<128>, 128, false, g6_128, d, h->d_dp, h->cur, h->cell_start, h->key_sorted, g_stage6, rng);
+    else if (rng) LAUNCH(k_pass_a4<true>, cdiv(count, PT4), PT4, d, h->d_dp, h->cur, h->cell_start, h->key_sorted, rng);
+    else LAUNCH(k_pass_a4<false>, cdiv(count, PT4), PT4, d, h->d_dp, h->cur, h->cell_start, h->key_sorted, rng);
     return SPHSM_OK;
 }
 // DIAG: ACC for the diagnostics download; EGM: the electrogram source Q (while electrograms are on)
 template <bool DIAG, bool EGM>
-static int launch_pass_b_as(sphsm_handle *h, const DevParams &d, int begin, int end, int hole_b, int hole_e, int count, uint32_t *nk, uint32_t *nr,
-                            uint32_t *ncnt, const int *rng) {
-    if (warp_path(h)) {
-        LAUNCH((k_pass_b4w<DIAG, EGM>), cdiv((long long)count * 32, PTW), PTW, d, h->cur, h->alt.P, h->cell_start, nk, nr, ncnt, count, rng);
-    } else if (g_pass_gen == 4) {
-        if (rng) LAUNCH((k_pass_b4<DIAG, true, EGM>), cdiv(count, PT4), PT4, d, h->d_dp, h->cur, h->alt.P, h->cell_start, h->key_sorted, nk, nr, ncnt, rng);
-        else LAUNCH((k_pass_b4<DIAG, false, EGM>), cdiv(count, PT4), PT4, d, h->d_dp, h->cur, h->alt.P, h->cell_start, h->key_sorted, nk, nr, ncnt, rng);
-    } else if (g_t6 == 64) {
-        const int grid = rng ? cdiv(count, 64) + 2 : grid6(begin, end, hole_b, hole_e, 64);
-        if (g_b_step6 == 4) LAUNCH6((k_pass_b6<64, 4, DIAG, EGM>), 64, true, grid, d, h->d_dp, h->cur, h->alt.P, h->cell_start, h->key_sorted, nk, nr, ncnt, g_stage6, rng);
-        else LAUNCH6((k_pass_b6<64, 2, DIAG, EGM>), 64, true, grid, d, h->d_dp, h->cur, h->alt.P, h->cell_start, h->key_sorted, nk, nr, ncnt, g_stage6, rng);
-    } else {
-        const int grid = rng ? cdiv(count, 128) + 2 : grid6(begin, end, hole_b, hole_e, 128);
-        if (g_b_step6 == 4) LAUNCH6((k_pass_b6<128, 4, DIAG, EGM>), 128, true, grid, d, h->d_dp, h->cur, h->alt.P, h->cell_start, h->key_sorted, nk, nr, ncnt, g_stage6, rng);
-        else LAUNCH6((k_pass_b6<128, 2, DIAG, EGM>), 128, true, grid, d, h->d_dp, h->cur, h->alt.P, h->cell_start, h->key_sorted, nk, nr, ncnt, g_stage6, rng);
-    }
+static int launch_pass_b_as(sphsm_handle *h, const DevParams &d, int count, uint32_t *nk, uint32_t *nr, uint32_t *ncnt, const int *rng) {
+    if (warp_path(h)) LAUNCH((k_pass_b4w<DIAG, EGM>), cdiv((long long)count * 32, PTW), PTW, d, h->cur, h->alt.P, h->cell_start, nk, nr, ncnt, count, rng);
+    else if (rng) LAUNCH((k_pass_b4<DIAG, true, EGM>), cdiv(count, PT4), PT4, d, h->d_dp, h->cur, h->alt.P, h->cell_start, h->key_sorted, nk, nr, ncnt, rng);
+    else LAUNCH((k_pass_b4<DIAG, false, EGM>), cdiv(count, PT4), PT4, d, h->d_dp, h->cur, h->alt.P, h->cell_start, h->key_sorted, nk, nr, ncnt, rng);
     return SPHSM_OK;
 }
 static int launch_pass_b(sphsm_handle *h, int begin, int end, bool diag, int hole_b = 0, int hole_e = 0, bool file_counts = false,
@@ -384,10 +338,8 @@ static int launch_pass_b(sphsm_handle *h, int begin, int end, bool diag, int hol
     DevParams d = h->dp;
     d.own_begin = begin; d.own_end = end; d.hole_begin = hole_b; d.hole_len = hole_e - hole_b;
     if (h->egm.on)
-        return diag ? launch_pass_b_as<true, true>(h, d, begin, end, hole_b, hole_e, count, nk, nr, ncnt, rng)
-                    : launch_pass_b_as<false, true>(h, d, begin, end, hole_b, hole_e, count, nk, nr, ncnt, rng);
-    return diag ? launch_pass_b_as<true, false>(h, d, begin, end, hole_b, hole_e, count, nk, nr, ncnt, rng)
-                : launch_pass_b_as<false, false>(h, d, begin, end, hole_b, hole_e, count, nk, nr, ncnt, rng);
+        return diag ? launch_pass_b_as<true, true>(h, d, count, nk, nr, ncnt, rng) : launch_pass_b_as<false, true>(h, d, count, nk, nr, ncnt, rng);
+    return diag ? launch_pass_b_as<true, false>(h, d, count, nk, nr, ncnt, rng) : launch_pass_b_as<false, false>(h, d, count, nk, nr, ncnt, rng);
 }
 
 // one fused step: grid, shape matching, pass A, pass B
@@ -515,7 +467,7 @@ static std::string step_signature(const sphsm_handle *h) {
     put(egm_f, sizeof(egm_f));
     const int egm_cfg[] = {(int)h->egm.on, h->egm.n_el, h->egm.rows, h->egm.grid};
     put(egm_cfg, sizeof(egm_cfg));
-    const int flags[] = {h->counts_ready, h->bounds_ready, h->sorted_buf, g_pass_gen, h->red_blocks, h->sort_passes, (int)h->grid_valid, (int)warp_path(h), g_stage6, g_t6, g_b_step6};
+    const int flags[] = {h->counts_ready, h->bounds_ready, h->sorted_buf, h->red_blocks, h->sort_passes, (int)h->grid_valid, (int)warp_path(h)};
     put(flags, sizeof(flags));
     return sig;
 }

@@ -39,7 +39,8 @@ def _ip(a):
 
 
 def tune(name: str, value: int):
-    """sphsm_tune: process-wide kernel-path switch ("pass", "stage6", "t6", "b_step6", "warp_path"); changes no result."""
+    """sphsm_tune: process-wide switch "warp_path" (1 | 0) or "x1_dynamic" (0 | 1); the first value is the default.
+    warp_path=0 changes the order of the floating-point sums on small dense sets."""
     lib = _capi.load()
     _capi.check(lib, None, lib.sphsm_tune(name.encode(), int(value)))
 

@@ -43,6 +43,23 @@ def test_default_params_match_reference_ctor():
     assert p.struct_size == __import__("ctypes").sizeof(_capi.Params)
 
 
+def test_tune_accepts_only_the_existing_switches():
+    """sphsm_tune (no device needed) takes "warp_path" and "x1_dynamic" at 0 / 1 and rejects every other name or value."""
+    lib = _capi.load()
+    err_invalid = -1  # SPHSM_ERR_INVALID
+    try:
+        for name in (b"warp_path", b"x1_dynamic"):
+            for value in (0, 1):
+                assert lib.sphsm_tune(name, value) == 0, (name, value)
+            for value in (-1, 2, 4, 64):
+                assert lib.sphsm_tune(name, value) == err_invalid, (name, value)
+        for name, value in ((b"pass", 4), (b"pass", 6), (b"stage6", 1), (b"t6", 128), (b"b_step6", 2), (b"no_such_switch", 0)):
+            assert lib.sphsm_tune(name, value) == err_invalid, (name, value)
+        assert lib.sphsm_tune(None, 0) == err_invalid
+    finally:
+        assert lib.sphsm_tune(b"warp_path", 1) == 0 and lib.sphsm_tune(b"x1_dynamic", 0) == 0  # the defaults
+
+
 def test_create_without_gpu_fails_loudly():
     """No CUDA device -> sphsm_create returns an error (no CPU fallback). Skipped where a GPU exists."""
     import ctypes as C

@@ -397,52 +397,3 @@ def test_midrun_fixation_matches_oracle(Sim, mode, parity_record):
             err = assert_close(f, got[f], want[f], params, tol=tol)
             parity_record("midrun_fixation", f"{mode}/step{step + 1}", f, err, tol)
     assert np.abs(want["predicted_vel"][newly]).max() > 1e-3  # the case is not vacuous: they were moving when they froze
-
-
-@pytest.mark.parametrize("case", ["jitter_lattice", "jitter_lattice_quadratic", "dense_mesh", "sparse_cloud"])
-def test_staged_matches_gathered(Sim, case):
-    """The block-staged neighbour passes (generation 6: stencil spans fetched into shared memory by bulk copies) visit the same
-    candidates in the same order with the same arithmetic as the gathered passes: every field of every particle is BIT-IDENTICAL
-    between the gathered generation 4, the staged kernels at 64 / 128 targets per block and 2 / 4 candidates per iteration, and the
-    staged kernels with staging refused for every block.  Covers blocks that stage (lattice), blocks too full to stage (the
-    reference's dense mesh through the thread-per-particle kernels) and key ranges too long to stage (sparse cloud)."""
-    from sph_sm_monodomain_b200.sim import tune
-
-    quadratic, warp = False, 1
-    if case.startswith("jitter_lattice"):
-        pos, world = inputs.lattice(64, 30, 30, jitter=0.05)
-        fixed, stim = inputs.lattice_masks(pos, 64, 8)
-        fixed, stim = fixed.astype(np.uint8), np.where(stim, np.float32(300), np.float32(0)).astype(np.float32)
-        quadratic = case.endswith("quadratic")
-    elif case == "dense_mesh":
-        g, _ = load_golden("cfg2_5211_wave")
-        pos, world, fixed, stim, warp = g["positions"], (1.5, 1.5, 1.5), g["init.fixed"].astype(np.uint8), g["init.stim"].astype(np.float32), 0
-    else:
-        rng = np.random.default_rng(7)
-        pos = (rng.random((20000, 3), dtype=np.float32) * np.float32(1.45) + np.float32(0.02)).astype(np.float32)
-        world, fixed = (1.5, 1.5, 1.5), np.zeros(20000, np.uint8)
-        stim = np.where(pos[:, 0] < 0.3, np.float32(300), np.float32(0)).astype(np.float32)
-    variants = [dict(**{"pass": 4}), dict(**{"pass": 6}, stage6=1, t6=128, b_step6=2), dict(**{"pass": 6}, stage6=1, t6=64, b_step6=4),
-                dict(**{"pass": 6}, stage6=1, t6=128, b_step6=4), dict(**{"pass": 6}, stage6=0, t6=128, b_step6=2)]
-    ref = None
-    try:
-        tune("warp_path", warp)
-        for v in variants:
-            for k, val in v.items():
-                tune(k, val)
-            s = Sim(capacity=len(pos), world=world, diagnostics=True)
-            s.Init_Fluid(pos)
-            s.set_masks(fixed, stim)
-            if quadratic:
-                s.flip_quadratic()
-            s.Animation(4)
-            p = s.particles()
-            s.close()
-            if ref is None:
-                ref = p
-            else:
-                bad = [f for f in FIELDS if not bits_equal(p[f], ref[f])]
-                assert not bad, (v, bad)
-    finally:
-        for k, val in (("pass", 4), ("stage6", 1), ("t6", 128), ("b_step6", 2), ("warp_path", 1)):
-            tune(k, val)

@@ -4,7 +4,7 @@ mkdir -p gpurun_out
 OUT=gpurun_out/sanitizer_r02.txt
 echo "# compute-sanitizer $(compute-sanitizer --version | head -1) on $(nvidia-smi --query-gpu=name --format=csv,noheader | head -1); cases = tools/sanitize_case.py" > $OUT
 for tool in memcheck racecheck synccheck; do
-  for c in thread warp radix staged slab3 strict io; do
+  for c in thread warp radix slab3 strict io; do
     timeout 600 compute-sanitizer --tool $tool --print-limit 5 python tools/sanitize_case.py $c > gpurun_out/san_${tool}_$c.log 2>&1
     rc=$?
     summary=$(grep -E "ERROR SUMMARY|RACECHECK SUMMARY" gpurun_out/san_${tool}_$c.log | tail -1)

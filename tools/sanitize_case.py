@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """One small scenario for compute-sanitizer (tools/gpu_sanitize.sh): a few steps through the C-ABI on a chosen kernel path.
-    python tools/sanitize_case.py thread|warp|radix|staged|slab3|strict|io"""
+    python tools/sanitize_case.py thread|warp|radix|slab3|strict|io"""
 import os
 import sys
 
@@ -8,16 +8,12 @@ import numpy as np
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from sph_sm_monodomain_b200 import LocalGroup, Sim, inputs, slabs  # noqa: E402
-from sph_sm_monodomain_b200.sim import tune  # noqa: E402
 
 case = sys.argv[1]
 G = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden")
-if case in ("thread", "radix", "staged", "strict", "io"):
+if case in ("thread", "radix", "strict", "io"):
     pos = inputs.init_cube_positions()  # 4913 particles: thread-per-particle kernels
-    kw = {}
-    if case == "staged":
-        tune("pass", 6)
-    sim = Sim(diagnostics=(case == "io"), strict=(case == "strict"), **kw)
+    sim = Sim(diagnostics=(case == "io"), strict=(case == "strict"))
     if case == "radix":
         p = sim.get_params()
         p.reserved[2] = 1  # LSD radix sort (decoupled look-back) instead of the counting sort
