@@ -52,7 +52,7 @@ struct sphsm_handle {
     cudaStream_t stream = nullptr;
     cudaStream_t launch_stream = nullptr;  // where LAUNCH enqueues: `stream`, except while the side chain below is built
     cudaStream_t side_stream = nullptr;    // slab step: moment sums + allreduce + solve run here, beside the sort
-    cudaEvent_t ev_fork = nullptr, ev_join = nullptr, ev_meta = nullptr, ev_bnd = nullptr, ev_int = nullptr;
+    cudaEvent_t ev_fork = nullptr, ev_join = nullptr, ev_bnd = nullptr, ev_int = nullptr;
     bool moments_forked = false;
     bool allreduce_pending = false;        // slab step: the forked sums still need their allreduce (issued after exchange 1 on a shared communicator)
     double meta_wait_us = 0.0;             // SPHSM_HOST_PROF: host time spent waiting for the plane boundaries
@@ -470,7 +470,6 @@ static int create_impl(const sphsm_params *p, sphsm_handle **out, sphsm_handle *
     }
     CU(cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming));
     CU(cudaEventCreateWithFlags(&h->ev_join, cudaEventDisableTiming));
-    CU(cudaEventCreateWithFlags(&h->ev_meta, cudaEventDisableTiming));
     CU(cudaStreamCreateWithFlags(&h->h2d_stream, cudaStreamNonBlocking));
     CU(cudaStreamCreateWithFlags(&h->d2h_stream, cudaStreamNonBlocking));
     for (cudaEvent_t *e : {&h->ev_in_ready, &h->ev_in_free, &h->ev_out_ready, &h->ev_out_done}) CU(cudaEventCreateWithFlags(e, cudaEventDisableTiming));
@@ -554,7 +553,6 @@ extern "C" int sphsm_destroy(sphsm_handle *h) {
     if (h->ev_join) cudaEventDestroy(h->ev_join);
     for (auto &gx : h->graphs) cudaGraphExecDestroy(gx.exec);
     h->graphs.clear();
-    if (h->ev_meta) cudaEventDestroy(h->ev_meta);
     for (cudaEvent_t e : {h->ev_in_ready, h->ev_in_free, h->ev_out_ready, h->ev_out_done})
         if (e) cudaEventDestroy(e);
     if (h->h2d_stream) cudaStreamDestroy(h->h2d_stream);

@@ -241,8 +241,9 @@ static int corrected_velocity(sphsm_handle *h, bool diag, GroupTimer *gt, int st
     const int keep_goal = n <= 1;  // projectPositions returned early: mGoalPos keeps its previous value
     if ((diag || keep_goal) && store == 7) h->goal_pv_stale = false;
     else if (!(diag || keep_goal)) h->goal_pv_stale = true;
-    if (diag || keep_goal) LAUNCH((k_goal_cvel<STRICT, true>), cdiv(n, 256), 256, h->dp, h->cur, h->sm, keep_goal, store);
-    else LAUNCH((k_goal_cvel<STRICT, false>), cdiv(n, 256), 256, h->dp, h->cur, h->sm, 0, store);
+    // the fast path comes here only with diag (sphsm_stage) or keep_goal (the single-particle step): one form of the kernel
+    if (STRICT && !(diag || keep_goal)) LAUNCH((k_goal_cvel<true, false>), cdiv(n, 256), 256, h->dp, h->cur, h->sm, 0, store);
+    else LAUNCH((k_goal_cvel<STRICT, true>), cdiv(n, 256), 256, h->dp, h->cur, h->sm, keep_goal, store);
     if (gt) gt->end_group(KG_GOAL);
     CU(cudaGetLastError());
     return SPHSM_OK;
@@ -294,7 +295,7 @@ static int run_stage(sphsm_handle *h, int stage) {
 // the fast-path neighbour passes over the owned slot range (count = own_end - own_begin)
 // Small particle sets (the reference's own ~5k-particle inputs) take one warp per particle (sphsm_pass4w.cuh).  The choice
 // follows the GLOBAL particle count, so that a slab rank and the single-GPU run of the same set use the same kernels (the
-// bit-level slab parity depends on identical summation order).  SPHSM_WARP_PATH=0 disables it, SPHSM_WARP_PATH_MAX moves the limit.
+// bit-level slab parity depends on identical summation order).  SPHSM_WARP_PATH=0 disables it.
 // The limit is a particle count because that is all the host knows; what actually decides is candidates per stencil row:
 // measured with the limit lifted, a 64k LATTICE (3-6 candidates per row, most lanes idle) runs pass A / B in 56 / 108 us on
 // this path against 16 / 21 us on the thread path, while the reference's meshes (45 per row) gain 10x.  Hence the second
@@ -302,9 +303,8 @@ static int run_stage(sphsm_handle *h, int stage) {
 // (note_host_positions; the reference's sets have 4.9-5.1, lattices of spacing 0.9 h have 1.4).
 static bool warp_path(const sphsm_handle *h) {
     if (!g_warp_path) return false;
-    static const int limit = getenv("SPHSM_WARP_PATH_MAX") ? atoi(getenv("SPHSM_WARP_PATH_MAX")) : WARP_PATH_MAX;
     const int n = h->dp.slab_on ? h->n_global : h->n;
-    if (n > limit || h->host_cells.empty()) return false;
+    if (n > WARP_PATH_MAX || h->host_cells.empty()) return false;
     return (double)n >= 3.0 * (double)h->host_cells.size();  // >= 3 particles per occupied cell: rows long enough for a warp
 }
 
@@ -354,40 +354,42 @@ static int fused_step(sphsm_handle *h) {
         CU(cudaMemcpyAsync(h->d_dp, &h->dp_uploaded, sizeof(DevParams), cudaMemcpyHostToDevice, h->stream));
     }
     GroupTimer gt(h);
-    if (!STRICT && n > 1) {
-        // sort -> shape-matching transform (slot-order independent) -> cell table + gather fused with stage 2's map
-        // the moment sums and the solve only read the not-yet-sorted arrays: they run on the side stream beside the sort
-        // and rejoin before the gather applies the transform (kept in line while the per-group timers are on)
-        const bool fork = !h->rest_dirty && !h->profiling;
-        if (fork) {
-            if (!h->dry_run) {
-                CU(cudaEventRecord(h->ev_fork, h->stream));
-                CU(cudaStreamWaitEvent(h->side_stream, h->ev_fork, 0));
-            }
-            h->launch_stream = h->side_stream;
-            rc = sm_transform_fast(h);
-            h->launch_stream = h->stream;
-            if (rc) return rc;
-            if (!h->dry_run) CU(cudaEventRecord(h->ev_join, h->side_stream));
-        }
-        if ((rc = grid_sort(h, &gt)) != 0) return rc;
-        if (fork) {
-            if (!h->dry_run) CU(cudaStreamWaitEvent(h->stream, h->ev_join, 0));
-        } else if ((rc = sm_transform_fast(h)) != 0) return rc;
-        gt.end_group(KG_MOMENTS);
-        if ((rc = grid_finish(h, &gt, diag ? 2 : 1)) != 0) return rc;
-    } else {
+    if constexpr (STRICT) {
         if ((rc = build_grid(h, &gt)) != 0) return rc;
-        if ((rc = corrected_velocity<STRICT>(h, diag, &gt)) != 0) return rc;
-    }
-    if (STRICT) {
-        LAUNCH((k_pass_a<STRICT, true, true>), cdiv(n, 128), 128, h->dp, h->cur, h->cell_start);
+        if ((rc = corrected_velocity<true>(h, diag, &gt)) != 0) return rc;
+        LAUNCH((k_pass_a<true, true, true>), cdiv(n, 128), 128, h->dp, h->cur, h->cell_start);
         gt.end_group(KG_PASS_A);
-        if (diag && h->egm.on) LAUNCH((k_pass_b<STRICT, PB_FUSED_DIAG | PB_EGM>), cdiv(n, 128), 128, h->dp, h->cur, h->alt.P, h->cell_start);
-        else if (diag) LAUNCH((k_pass_b<STRICT, PB_FUSED_DIAG>), cdiv(n, 128), 128, h->dp, h->cur, h->alt.P, h->cell_start);
-        else if (h->egm.on) LAUNCH((k_pass_b<STRICT, PB_FUSED | PB_EGM>), cdiv(n, 128), 128, h->dp, h->cur, h->alt.P, h->cell_start);
-        else LAUNCH((k_pass_b<STRICT, PB_FUSED>), cdiv(n, 128), 128, h->dp, h->cur, h->alt.P, h->cell_start);
+        if (diag && h->egm.on) LAUNCH((k_pass_b<true, PB_FUSED_DIAG | PB_EGM>), cdiv(n, 128), 128, h->dp, h->cur, h->alt.P, h->cell_start);
+        else if (diag) LAUNCH((k_pass_b<true, PB_FUSED_DIAG>), cdiv(n, 128), 128, h->dp, h->cur, h->alt.P, h->cell_start);
+        else if (h->egm.on) LAUNCH((k_pass_b<true, PB_FUSED | PB_EGM>), cdiv(n, 128), 128, h->dp, h->cur, h->alt.P, h->cell_start);
+        else LAUNCH((k_pass_b<true, PB_FUSED>), cdiv(n, 128), 128, h->dp, h->cur, h->alt.P, h->cell_start);
     } else {
+        if (n > 1) {
+            // sort -> shape-matching transform (slot-order independent) -> cell table + gather fused with stage 2's map
+            // the moment sums and the solve only read the not-yet-sorted arrays: they run on the side stream beside the sort
+            // and rejoin before the gather applies the transform (kept in line while the per-group timers are on)
+            const bool fork = !h->rest_dirty && !h->profiling;
+            if (fork) {
+                if (!h->dry_run) {
+                    CU(cudaEventRecord(h->ev_fork, h->stream));
+                    CU(cudaStreamWaitEvent(h->side_stream, h->ev_fork, 0));
+                }
+                h->launch_stream = h->side_stream;
+                rc = sm_transform_fast(h);
+                h->launch_stream = h->stream;
+                if (rc) return rc;
+                if (!h->dry_run) CU(cudaEventRecord(h->ev_join, h->side_stream));
+            }
+            if ((rc = grid_sort(h, &gt)) != 0) return rc;
+            if (fork) {
+                if (!h->dry_run) CU(cudaStreamWaitEvent(h->stream, h->ev_join, 0));
+            } else if ((rc = sm_transform_fast(h)) != 0) return rc;
+            gt.end_group(KG_MOMENTS);
+            if ((rc = grid_finish(h, &gt, diag ? 2 : 1)) != 0) return rc;
+        } else {
+            if ((rc = build_grid(h, &gt)) != 0) return rc;
+            if ((rc = corrected_velocity<false>(h, diag, &gt)) != 0) return rc;
+        }
         if ((rc = launch_pass_a(h, 0, n)) != 0) return rc;  // single GPU: own range = [0, n)
         gt.end_group(KG_PASS_A);
         // the counting sort of the NEXT step starts inside pass B: each thread files the key / rank / count of the position it

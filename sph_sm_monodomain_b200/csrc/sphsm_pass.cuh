@@ -4,8 +4,9 @@
 //                                   one sweep over the 27-cell stencil
 //   k_pass_b<STRICT, MODE>          ionic cell model (cpp:575-593) + pressure/viscosity force + SPH Laplacian of Vm
 //                                   (cpp:515-573) + integration, Vm clamp and walls (cpp:598-651) in one sweep;
-//                                   MODE selects the staged variants (force only) used by sphsm_stage(); MODE | PB_EGM
-//                                   also stores the electrogram source vol * L (sphsm_egm.cuh)
+//                                   MODE selects the fused sweep of the strict step or the force-only stage 6 of
+//                                   sphsm_stage() (the only mode of the fast form: the fast step runs sphsm_pass4*.cuh);
+//                                   MODE | PB_EGM also stores the electrogram source vol * L (sphsm_egm.cuh)
 //   k_cell_model, k_update          the stand-alone per-particle stages for sphsm_stage()
 // v1 mapping: one thread per particle over the cell-sorted SoA arrays; neighbouring threads sit in the same or
 // adjacent cells, so their float4 gathers hit the same L1 lines.
@@ -127,6 +128,7 @@ __global__ void __launch_bounds__(128) k_pass_b(const __grid_constant__ DevParam
                                                 const int *__restrict__ cell_start) {
     using A = Ar<STRICT>;
     constexpr int MODE = MODE_EGM & ~PB_EGM;
+    static_assert(STRICT || MODE == PB_FORCE_ONLY, "the fast step runs k_pass_b4 / k_pass_b4w; only sphsm_stage's force pass is fast here");
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= p.n) return;
     const float4 pi = a.P[i];

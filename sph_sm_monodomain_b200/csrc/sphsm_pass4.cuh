@@ -21,10 +21,7 @@
 
 namespace sphsm {
 
-#ifndef SPHSM_LIST_K
-#define SPHSM_LIST_K 16
-#endif
-constexpr int LIST_K = SPHSM_LIST_K;  // in-range list entries per lane between drains
+constexpr int LIST_K = 16;  // in-range list entries per lane between drains (12 and 14 measured slower: DESIGN.md §4)
 
 __device__ __forceinline__ float rsqrt_ftz(float x) {
     float y;
@@ -77,16 +74,10 @@ __device__ __forceinline__ int list_get(unsigned addr) {
     asm volatile("ld.shared.b32 %0, [%1];" : "=r"(v) : "r"(addr) : "memory");
     return v;
 }
-#ifndef SPHSM_PT4
-#define SPHSM_PT4 128  // measured at 8M (pass A / pass B us): 64: 484 / 689, 128: 469 / 678, 256: 497 / 692, 512: 523 / 720
-#endif
-constexpr int PT4 = SPHSM_PT4;        // threads per block of the generation-4 passes
-#ifndef SPHSM_A_MINB
-#define SPHSM_A_MINB 9  // resident blocks per SM pass A / pass B are compiled for: 56 / 64 registers (measured in round 2 against 8 / 7: see DESIGN.md)
-#endif
-#ifndef SPHSM_B_MINB
-#define SPHSM_B_MINB 8
-#endif
+// threads per block of the generation-4 passes, measured at 8M (pass A / pass B us): 64: 484 / 689, 128: 469 / 678, 256: 497 / 692, 512: 523 / 720
+constexpr int PT4 = 128;
+// resident blocks per SM pass A / pass B are compiled for: 56 / 64 registers (measured in round 2 against 8 / 7: see DESIGN.md)
+constexpr int A_MINB = 9, B_MINB = 8;
 constexpr unsigned LSTEP = 4u * PT4;  // bytes between consecutive entries of one lane
 // Likewise a gathered array's base pointer: `pinned(ptr, zero)` is ptr + 0 with the zero coming from global memory, formed
 // in PTX so that neither the front end (which would fold it into the index) nor ptxas (which would re-load the kernel
@@ -243,7 +234,7 @@ __device__ __forceinline__ void pass_a4_one(const DevParams &p, const DevParams 
 // RNG: the launch range comes from device memory (slab step).  A template parameter, not a run-time test: with the test compiled
 // in, the single-GPU kernel kept 48 bytes of spills at its 56 registers and lost 10 % (ncu r02: 520 us against 470).
 template <bool RNG>
-__global__ void __launch_bounds__(PT4, SPHSM_A_MINB) k_pass_a4(const __grid_constant__ DevParams p, const DevParams *__restrict__ g, Arrays a,
+__global__ void __launch_bounds__(PT4, A_MINB) k_pass_a4(const __grid_constant__ DevParams p, const DevParams *__restrict__ g, Arrays a,
                                                 const int *__restrict__ cell_start, const uint32_t *__restrict__ skey, const int *__restrict__ rng) {
     __shared__ int s_list[LIST_K * PT4];
     int i;
@@ -262,21 +253,10 @@ __global__ void __launch_bounds__(PT4, SPHSM_A_MINB) k_pass_a4(const __grid_cons
 
 // ---------------------------------------------------------------------------------------------------
 // Update_Properties (cpp:602-649) with reciprocals on the velocity / position side.  The voltage side of the step (ionic
-// model with its double promotions, Inter_Vm, the Vm update) keeps the reference's exact operations by default: Vm then
-// stays BIT-IDENTICAL to the reference wherever the Laplacian vanishes (both Resources/*.csv configs as main.cpp runs
-// them), and the excitable dynamics amplify rounding differences (cfg2 wave, |dVm| max at step 200: 2.8e-2 exact,
-// 6.7e-2 with -DSPHSM_FAST_ODE=1, for 22 us of 717 at 8M).
-#ifndef SPHSM_FAST_ODE
-#define SPHSM_FAST_ODE 0
-#endif
-__device__ __forceinline__ void cell_model_fast(const DevParams &p, float Vm, float inv_mass, float &Iion, float &w) {
-    const float u = (Vm - p.Vr) / p.fh_denom;
-    const float c1 = p.C1 * u * (u - p.fh_asd);
-    const float t = fmaf(c1, u - 1.0f, p.C2 * w);
-    const float dtm = p.dt * inv_mass;
-    Iion = fmaf(dtm, t, Iion);
-    w = fmaf(dtm * p.C3, u - p.C4 * w, w);
-}
+// model with its double promotions, Inter_Vm, the Vm update) keeps the reference's exact operations: Vm then stays
+// BIT-IDENTICAL to the reference wherever the Laplacian vanishes (both Resources/*.csv configs as main.cpp runs them), and
+// the excitable dynamics amplify rounding differences (cfg2 wave, |dVm| max at step 200: 2.8e-2 exact, 6.7e-2 with a float
+// ionic model, which saved 22 us of 717 at 8M: DESIGN.md §4).
 __device__ __forceinline__ void integrate_fast(const DevParams &p, bool fixed, float dtm, float ivx, float ivy, float ivz, float ax, float ay, float az,
                                                float inter_vm, float mass, float &x, float &y, float &z, float &vx, float &vy, float &vz, float &Vm) {
     if (!fixed) {
@@ -287,7 +267,7 @@ __device__ __forceinline__ void integrate_fast(const DevParams &p, bool fixed, f
         y = fmaf(vy, p.dt, y);
         z = fmaf(vz, p.dt, z);
     }
-    Vm = SPHSM_FAST_ODE ? fmaf(inter_vm, dtm, Vm) : Vm + div_rn_z(inter_vm * p.dt, mass);  // cpp:612
+    Vm = Vm + div_rn_z(inter_vm * p.dt, mass);  // cpp:612
     Vm = fminf(fmaxf(Vm, -p.max_voltage), p.max_voltage);
     // walls (cpp:620-646); the final bounds.clamp (m3Bounds.h:84-88) cannot move a position that passed them
     if (x < 0.0f) { vx *= p.wall_hit; x = 0.0f; }
@@ -317,7 +297,7 @@ __device__ __forceinline__ void pass_b_finish(const DevParams &p, const Arrays &
     az *= inv_dens;
     // cpp:571: Inter_Vm += (sigma/(Beta*Cm))*Inter_Vm - ((Iion - stim*dt/mass)/Cm)   (the += form, Q9)
     const float dtm = p.dt * inv_mass;
-    const float ivm = SPHSM_FAST_ODE ? L + (p.diff_coef * L - (e4.y - e4.w * dtm) / p.Cm) : L + (p.diff_coef * L - (e4.y - div_rn_z(e4.w * p.dt, pi.w)) / p.Cm);
+    const float ivm = L + (p.diff_coef * L - (e4.y - div_rn_z(e4.w * p.dt, pi.w)) / p.Cm);
     if (DIAG) a.ACC[i] = make_float4(ax, ay, az, ivm);
     if (EGM) a.Q[i] = vi.w * L;
     float x = pi.x, y = pi.y, z = pi.z;
@@ -333,9 +313,6 @@ __device__ __forceinline__ void pass_b_finish(const DevParams &p, const Arrays &
     }
 }
 
-#ifndef SPHSM_B_STEP
-#define SPHSM_B_STEP 2  // candidates per unchecked iteration of pass B phase 1 (2 or 4; 4 needs 72 registers and measured 686 us against 678)
-#endif
 // pass B: ionic cell model + pressure / viscosity force + SPH Laplacian of Vm + integration and walls
 // (reference cpp:575-593, 515-573, 598-651).  PB = (pos.xyz, Vm) is the neighbour record of this pass.
 // cell_count != nullptr: the thread also files its particle's NEW position for the next step's counting sort (key, provisional
@@ -352,8 +329,7 @@ __device__ __forceinline__ void pass_b4_one(const DevParams &p, const DevParams 
     const float pres_i = si.x;
     const float Vm_i = e4.x;
     const float inv_mass = rcp_ftz(pi.w);
-    if (SPHSM_FAST_ODE) cell_model_fast(p, e4.x, inv_mass, e4.y, e4.z);
-    else cell_model<false>(p, e4.x, pi.w, e4.y, e4.z);
+    cell_model<false>(p, e4.x, pi.w, e4.y, e4.z);
 
     const int z0 = g->zero;  // == 0, loaded from global: what is derived from it stays in registers (see list_put)
     const float4 *__restrict__ PB = pinned(a.PB, z0);
@@ -383,20 +359,9 @@ __device__ __forceinline__ void pass_b4_one(const DevParams &p, const DevParams 
             acc = on ? t : acc;
             return on && r2 <= sp2;
         };
-        sweep4<SPHSM_B_STEP>(
+        // two candidates per iteration (four, as in pass A, need 72 registers and measured 686 us against 678: DESIGN.md §4)
+        sweep4<2>(
             p, cell_start, ga, gagb, key, lbase, lofs,
-#if SPHSM_B_STEP == 4
-            [&](int j, int e, unsigned &lo) {
-                const float4 p0 = __ldg(PB + j), p1 = __ldg(PB + j + 1), p2 = __ldg(PB + j + 2), p3 = __ldg(PB + j + 3);
-                const float v0 = __ldg(VN + j), v1 = __ldg(VN + j + 1), v2 = __ldg(VN + j + 2), v3 = __ldg(VN + j + 3);
-                const bool i0 = cand(p0, v0, true, L), i1 = cand(p1, v1, j + 1 < e, L1);
-                const bool i2 = cand(p2, v2, j + 2 < e, L), i3 = cand(p3, v3, j + 3 < e, L1);
-                if (i0) { list_put(lo, j); lo += LSTEP; }
-                if (i1) { list_put(lo, j + 1); lo += LSTEP; }
-                if (i2) { list_put(lo, j + 2); lo += LSTEP; }
-                if (i3) { list_put(lo, j + 3); lo += LSTEP; }
-            },
-#else
             [&](int j, bool two, unsigned &lo) {
                 const float4 p0 = __ldg(PB + j), p1 = __ldg(PB + j + 1);
                 const float v0 = __ldg(VN + j), v1 = __ldg(VN + j + 1);
@@ -409,7 +374,6 @@ __device__ __forceinline__ void pass_b4_one(const DevParams &p, const DevParams 
                     lo += LSTEP;
                 }
             },
-#endif
             [&](int j, unsigned &lo) {
                 if (cand(__ldg(PB + j), __ldg(VN + j), true, L)) {
                     list_put(lo, j);
@@ -443,7 +407,7 @@ __device__ __forceinline__ void pass_b4_one(const DevParams &p, const DevParams 
     pass_b_finish<DIAG, EGM>(p, a, Pout, i, pi, vi, e4, si.y, fixed, ax, ay, az, L + L1, inv_mass, next_keys, next_rank, cell_count);
 }
 template <bool DIAG, bool RNG, bool EGM>
-__global__ void __launch_bounds__(PT4, SPHSM_B_MINB) k_pass_b4(const __grid_constant__ DevParams p, const DevParams *__restrict__ g, Arrays a,
+__global__ void __launch_bounds__(PT4, B_MINB) k_pass_b4(const __grid_constant__ DevParams p, const DevParams *__restrict__ g, Arrays a,
                                                 float4 *__restrict__ Pout, const int *__restrict__ cell_start, const uint32_t *__restrict__ skey,
                                                 uint32_t *__restrict__ next_keys, uint32_t *__restrict__ next_rank, uint32_t *__restrict__ cell_count,
                                                 const int *__restrict__ rng) {

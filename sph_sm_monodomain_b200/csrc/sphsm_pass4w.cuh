@@ -100,8 +100,7 @@ __global__ void __launch_bounds__(PTW) k_pass_b4w(const __grid_constant__ DevPar
     const float pres_i = si.x;
     const float Vm_i = e4.x;
     const float inv_mass = rcp_ftz(pi.w);
-    if (SPHSM_FAST_ODE) cell_model_fast(p, e4.x, inv_mass, e4.y, e4.z);
-    else cell_model<false>(p, e4.x, pi.w, e4.y, e4.z);
+    cell_model<false>(p, e4.x, pi.w, e4.y, e4.z);
 
     const float4 *__restrict__ PB = a.PB;
     const float4 *__restrict__ V = a.V;

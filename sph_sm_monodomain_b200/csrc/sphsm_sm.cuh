@@ -262,22 +262,6 @@ __global__ void __launch_bounds__(256) k_rest_pass2(const __grid_constant__ DevP
     }
     block_reduce_store<9>(acc, partial + ((size_t)blockIdx.y * gridDim.x + blockIdx.x) * 9);
 }
-// fixed-order sum of per-block partials: totals[k] = sum_b partial[b*NACC + k]
-__global__ void __launch_bounds__(256) k_sum_partials(const double *__restrict__ partial, int blocks, int nacc, double *totals) {
-    __shared__ double s[256];
-    for (int k = 0; k < nacc; k++) {
-        double v = 0.0;
-        for (int b = threadIdx.x; b < blocks; b += 256) v += partial[(size_t)b * nacc + k];
-        s[threadIdx.x] = v;
-        __syncthreads();
-        for (int o = 128; o > 0; o >>= 1) {
-            if (threadIdx.x < o) s[threadIdx.x] += s[threadIdx.x + o];
-            __syncthreads();
-        }
-        if (threadIdx.x == 0) totals[k] = s[0];
-        __syncthreads();
-    }
-}
 __global__ void k_rest_finalize1(const double *__restrict__ tot, SmState *sm) {
     sm->Mfix = tot[0];
     sm->M = tot[1];
