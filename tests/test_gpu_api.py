@@ -184,8 +184,9 @@ def test_walls_reflect_and_clamp(Sim):
 # ---- properties at sizes the oracle cannot reach ----------------------------------------------------------------
 @pytest.mark.parametrize("n,world", [(1_000_000, (3.68, 3.68, 3.68)), (300_000, (18.52, 4.6, 4.6))])
 def test_large_random_cloud_grid_properties(Sim, n, world):
-    """Radix sort + cell table at 1M particles / up to 6M cells: the CSR is a permutation, every particle sits in the
-    bucket numpy computes for it, buckets are ascending, and sampled candidate sets equal brute force."""
+    """Cell table of large random clouds: 1M particles in 0.8M padded cells take the counting sort, 300k particles in 6.3M
+    padded cells the three-pass LSD radix sort.  The CSR is a permutation, every particle sits in the bucket numpy computes for
+    it, buckets are ascending, and sampled candidate sets equal brute force."""
     rng = np.random.Generator(np.random.PCG64(17))
     w = np.asarray(world, np.float32)
     pos = (rng.random((n, 3), dtype=np.float32) * (w - np.float32(0.001))).astype(np.float32)

@@ -34,12 +34,18 @@ def pres_is_defined(step, stage):
 
 
 # ---- the three protocols; each drives every simulation given in lockstep ------------------------------------------------
-def random_cloud(backends, seed, quadratic, volume):
-    """Yields (sims, step, stage) after every stage of CLOUD_STEPS steps; stimulation off after step 6."""
+# A back end is an oracle back-end name or a factory called with the CpuSim keyword arguments (the GPU tests pass Sim).
+def make_sim(backend, **kw):
+    return CpuSim(backend, **kw) if isinstance(backend, str) else backend(**kw)
+
+
+def random_cloud(backends, seed, quadratic, volume, fused=False):
+    """Yields (sims, step, stage) after every stage of CLOUD_STEPS steps; stimulation off after step 6.  fused: one
+    Animation(1) per step instead of the seven stages, yielding (sims, step, 7)."""
     rng = np.random.Generator(np.random.PCG64(seed))
     n = 1500
     pos = (rng.random((n, 3), dtype=np.float32) * np.float32(0.5) + np.float32(0.4)).astype(np.float32)
-    sims = [CpuSim(b) for b in backends]
+    sims = [make_sim(b) for b in backends]
     for s in sims:
         s.Init_Fluid(pos)
         s.set_stim((0.6, 0.6, 0.6), 0.02, 300.0)
@@ -49,9 +55,9 @@ def random_cloud(backends, seed, quadratic, volume):
         if not volume:
             s.flip_volume()
     for step in range(CLOUD_STEPS):
-        for st in range(1, 8):
+        for st in (7,) if fused else range(1, 8):
             for s in sims:
-                s.stage(st)
+                s.Animation(1) if fused else s.stage(st)
             yield sims, step, st
         if step == 6:
             for s in sims:
@@ -64,7 +70,7 @@ def walls(backends):
     n = 600
     pos = (rng.random((n, 3), dtype=np.float32) * np.float32(1.5)).astype(np.float32)
     vel = (rng.standard_normal((n, 3)) * 40).astype(np.float32)
-    sims = [CpuSim(b) for b in backends]
+    sims = [make_sim(b) for b in backends]
     for s in sims:
         s.Init_Fluid(pos)
         s.set_fields(vel=vel, stim=np.full(n, 300, np.float32))
@@ -75,7 +81,7 @@ def walls(backends):
 def lifted_world(backends):
     pos, world = inputs.lattice(14, 9, 11, jitter=0.1, seed=5)
     fixed, stim = inputs.lattice_masks(pos, 14, 3)
-    sims = [CpuSim(b, capacity=len(pos), world=world) for b in backends]
+    sims = [make_sim(b, capacity=len(pos), world=world) for b in backends]
     for s in sims:
         s.Init_Fluid(pos)
         s.set_fields(fixed=fixed, stim=np.where(stim, 300, 0).astype(np.float32))
